@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the SmartStart hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Headline metric: NND-MPC rollout-steps/s; the second half of
 BASELINE.json's metric, KDE kernel-evals/s, is reported in the same line under "kde".
@@ -48,6 +48,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 FLOP_PER_STEP = {2: 505_000, 3: 507_000}      # SURVEY 8(d): 2*[(d+da)h + h^2 + h d], h=500
 K_PER_GPU = 131_072
@@ -124,6 +125,13 @@ def shared_config(world):
     """`config` of the JSON line: identical keys and values in both arms (ours / --impl reference)."""
     return {"workload": workload_name(), "K_per_gpu": K_PER_GPU, "K_total": K_PER_GPU * world, "H": HORIZON,
             "mlp": "2x500", "d": 3, "da": 1, "penalty_mode": "reference", "gamma": .75, "horizontal_penalty_factor": .5}
+
+
+def dump_decision(out_dir, res):
+    """--dump-outputs: the arrays an MPC decision hands its caller, one float64 .npy each (scalars as shape (1,))."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("best_k", "best_score", "best_sequence", "best_path"):
+        np.save(os.path.join(out_dir, name + ".npy"), np.array(res[name], dtype=np.float64, ndmin=1))
 
 
 class ClockSampler(threading.Thread):
@@ -496,7 +504,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-step", action="store_true", help="reference arm: skip the full K=131072 step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed MPC decision returned (best_k, best_score, "
+                         "best_sequence, best_path) as DIR/<name>.npy in float64; the inputs depend only on the "
+                         "arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args, guard)
@@ -559,10 +575,12 @@ def main():
     half = max(3, args.steps // 2)
     precision = "bf16_tc" if eng.tc_supported() else "fp32"
     rollout_ms = []
+    last_decision = {}
 
     def mpc_step(i):
-        planner.plan(wl["state"], 0, K=K_total, H=HORIZON, seed=1000 + i, act_low=wl["low"], act_high=wl["high"],
-                     penalty_mode="reference", precision=precision, want_path=True)
+        last_decision["res"] = planner.plan(wl["state"], 0, K=K_total, H=HORIZON, seed=1000 + i, act_low=wl["low"],
+                                            act_high=wl["high"], penalty_mode="reference", precision=precision,
+                                            want_path=True)
         if i > 0:
             rollout_ms.append(dict(eng.last_timings()).get("mpc_rollout", 0.0))
 
@@ -577,6 +595,8 @@ def main():
     launches = eng.launch_count() - launches0
     ms_per_step = ms_total / args.steps
     value = K_total * HORIZON / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:         # every rank returns the same decision
+        dump_decision(args.dump_outputs, last_decision["res"])
 
     # ---- e2e through the plugin call: NND_MB_agent.get_best_sim_actions -------------------------
     np.random.seed(1234)                      # identical on every rank (lock-step agents)

@@ -1,6 +1,6 @@
 """Development helper: device time per Adam step of the trainer (row f1)."""
-import sys, time, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import bench
 from oracle import dyn_train_oracle as dto
 from smartstartcontinuous_b200.engine import Engine
