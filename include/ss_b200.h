@@ -55,7 +55,11 @@ enum {
     SS_PRECISION_FP32 = 0,     /* FP32 FFMA everywhere (SIMT kernel; parity mode)            */
     SS_PRECISION_BF16_TC = 1,  /* hidden x hidden layers on tcgen05 (BF16 in, FP32 accumulate
                                   in TMEM); first/last layer, state and scoring in FP32      */
-    SS_PRECISION_AUTO = 2      /* BF16_TC when the shape is supported, else FP32             */
+    SS_PRECISION_AUTO = 2,     /* BF16_TC when the shape is supported, else FP32             */
+    SS_PRECISION_FP64 = 3      /* everything in float64 in the reference's element-wise order
+                                  (DFMA rollout, float64 scores and arg-max): the reference's
+                                  decision up to the summation order of GEMMs and reductions;
+                                  AUTO never selects it                                       */
 };
 
 /* ---- context --------------------------------------------------------------------- */
@@ -141,7 +145,7 @@ int ss_mpc_set_plan(ss_ctx* ctx, const double* desired_states, int W,
  *                       sampled on the device with Philox4x32-10(seed) indexed by the GLOBAL
  *                       sequence number, uniform in [act_low, act_high) like npr.uniform.
  *   out_best_k          GLOBAL index of the first maximum score on this shard
- *   out_best_sequence   [H, da], out_best_path [H+1, d] (rolled out in FP32), out_scores [K_local]
+ *   out_best_sequence   [H, da], out_best_path [H+1, d] (rolled out in FP32; float64 with SS_PRECISION_FP64), out_scores [K_local]
  *                       (nullable)
  * In SS_PENALTY_REFERENCE mode with K_global != K_local use the three-call form below so the
  * per-time-step projection sums can be all-reduced across GPUs.
@@ -255,7 +259,8 @@ int ss_py_random_sample(uint32_t* mt_state, int* mt_index, int64_t first, int64_
 int ss_mpc_tc_supported(ss_ctx* ctx);
 /* rollout kernel of the last ss_mpc_rollout: 0 = FP32 SIMT, 1 = tcgen05 CTA pairs (mpc_tc.cu), 2 = tcgen05
  * 4-CTA clusters with the hidden layer split over the cluster (small batches, mpc_tc_quad.cu), 3 = FP32 thread per
- * sequence (one hidden layer of <= 64 units, the reference's default 1 x 32 model); -1 = none */
+ * sequence (one hidden layer of <= 64 units, the reference's default 1 x 32 model), 4 = float64 (SS_PRECISION_FP64,
+ * mpc_fp64.cu); -1 = none */
 int ss_mpc_last_kernel(ss_ctx* ctx);
 
 /* ---- dynamics-model training on the device (SURVEY 8f, row f1) ------------------------------

@@ -10,7 +10,7 @@ LIB_PATH = os.path.join(HERE, "libss_b200.so")
 
 SS_OK, SS_EINVAL, SS_ECUDA, SS_ESINGULAR, SS_ESTATE, SS_EUNSUPPORTED = 0, -1, -2, -3, -4, -5
 PENALTY_REFERENCE, PENALTY_PER_SAMPLE = 0, 1
-PRECISION_FP32, PRECISION_BF16_TC, PRECISION_AUTO = 0, 1, 2
+PRECISION_FP32, PRECISION_BF16_TC, PRECISION_AUTO, PRECISION_FP64 = 0, 1, 2, 3
 
 _c_double_p = C.POINTER(C.c_double)
 _c_float_p = C.POINTER(C.c_float)

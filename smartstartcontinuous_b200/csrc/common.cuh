@@ -63,6 +63,13 @@ struct MpcNorm {
     float mean_z[SS_MAX_D], std_z[SS_MAX_D];
 };
 
+// the caller's float64 statistics as they are (SS_PRECISION_FP64 divides by the standard deviations)
+struct MpcNorm64 {
+    double mean_x[SS_MAX_D], std_x[SS_MAX_D];
+    double mean_y[SS_MAX_DA], std_y[SS_MAX_DA];
+    double mean_z[SS_MAX_D], std_z[SS_MAX_D];
+};
+
 struct ActionSource {
     const double* host_actions;  // device copy of host-provided [K_local, H, da] doubles, or null
     uint64_t seed;
@@ -153,6 +160,8 @@ struct ss_ctx {
     int tc_hp = 0;
     int tc_quad_clusters = -1;         // co-resident 4-CTA clusters of the small-batch kernel (-1: not probed)
     std::vector<std::vector<double>> hw, hb;   // host copies of the float64 parameters
+    std::vector<DevBuf> w64, b64;      // padded float64 weights / biases (SS_PRECISION_FP64), same layout as w32 / b32
+    MpcNorm64 norm64;
     // ---- dynamics-model training on the device (dyn_train.cu): FP32 master parameters, Adam moments,
     // both training sets, per-batch activations
     DevBuf dyn_params, dyn_m, dyn_v, dyn_x[2], dyn_z[2], dyn_act, dyn_scratch, dyn_idx, dyn_losses;
@@ -167,20 +176,27 @@ struct ss_ctx {
     int W = 0;
     DevBuf plan_ds, plan_dl;           // fp32 [W][d], [W]
     float inv_radii[SS_MAX_D];
+    DevBuf plan_ds64, plan_dl64;       // float64 copies for SS_PRECISION_FP64
+    double radii64[SS_MAX_D];
     // ---- MPC run state
     DevBuf mpc_actions64, mpc_states, mpc_scores, mpc_partial_sums, mpc_sums, mpc_block_best,
         mpc_result, mpc_replay, mpc_sampled, mpc_package;
     double gpow_gamma = -1.0;          // gamma^t table currently resident in mpc_replay
     int gpow_T = 0;
+    // SS_PRECISION_FP64: trajectory rows [T][K][d + 1], scores, and [gamma^t (T) | replay rows T x (d + 1)]
+    DevBuf mpc_states64, mpc_scores64, mpc_misc64;
+    double gpow64_gamma = -1.0;
+    int gpow64_T = 0;
     struct {
         bool valid = false;
         int64_t K_local = 0, k_offset = 0, K_global = 0;
         int H = 0, wp_index = 0, penalty_mode = 0, precision = 0;
         double gamma = 0, hpf = 0;
         float state[SS_MAX_D];
+        double state64[SS_MAX_D];
         ActionSource act;
         bool states_stored = false;
-        int kernel = 0;                // rollout kernel of this decision: 0 FP32 SIMT, 1 tcgen05 CTA pairs, 2 tcgen05 4-CTA clusters
+        int kernel = 0;                // rollout kernel of this decision (ss_mpc_last_kernel)
         bool finished = false;         // the reference-mode penalty pass has rewritten the scores
         bool peer_sums = false;        // the projection sums were all-reduced over peer memory
         int sum_blocks = 0;

@@ -656,6 +656,13 @@ extern "C" int ss_dyn_commit(ss_ctx* c) {
                                                                     out_pad, c->w32[l].as<float>(), c->b32[l].as<float>());
         c->launches++;
     }
+    // the float64 copies of SS_PRECISION_FP64 roll out the same (widened) parameters Dyn_Model.export() returns
+    for (int l = 0; l <= y.L; ++l) {
+        const int out_pad = l == y.L ? (c->d + 7) / 8 * 8 : c->h_pad;
+        int rc = mpc_fp64_widen(c, P + y.w_off[l], P + y.b_off[l], y.in[l], y.out[l], out_pad, c->w64[l].as<double>(),
+                                c->b64[l].as<double>());
+        if (rc) return rc;
+    }
     if (c->tc_ready) {
         TcGeom g;
         std::memset(&g, 0, sizeof(g));

@@ -5,6 +5,8 @@
 //   ss_mpc_rollout    phase A: sample/fetch actions, roll the MLP for H steps, score
 //   ss_mpc_finish     phase B (reference penalty) + arg-max
 //   ss_mpc_replay     re-roll the winner for best_sequence / best_path (NND_MB_agent.py:516-518)
+// SS_PRECISION_FP64 keeps its own float64 copies of the model and the plan and its own rows / scores buffers
+// (mpc_fp64.cu, the float64 tail of mpc_score.cu); the projection sums and the package are shared.
 #include <atomic>
 #include <cstdlib>
 #include <cstring>
@@ -75,6 +77,32 @@ PlanView make_plan_view(ss_ctx* c, const float* gpow, double gamma, double hpf) 
     return p;
 }
 
+Plan64 make_plan64(ss_ctx* c, double gamma, double hpf) {
+    Plan64 p;
+    p.ds = c->plan_ds64.as<double>();
+    p.dl = c->plan_dl64.as<double>();
+    p.gpow = c->mpc_misc64.as<double>();
+    p.W = c->W;
+    p.d = c->d;
+    for (int j = 0; j < SS_MAX_D; ++j) p.r[j] = c->radii64[j];
+    p.hpf = hpf;
+    p.gamma = gamma;
+    return p;
+}
+
+// float64 rows of the fp64 replay (after the gamma^t table)
+double* misc64_rows(ss_ctx* c) { return c->mpc_misc64.as<double>() + (c->run.H + 2) / 2 * 2; }
+
+void fill_model64_args(ss_ctx* c, Rollout64Args& a) {
+    for (int l = 0; l <= c->L; ++l) {
+        a.w[l] = c->w64[l].as<double>();
+        a.b[l] = c->b64[l].as<double>();
+    }
+    a.d = c->d; a.da = c->da; a.L = c->L; a.h = c->h;
+    a.din_pad = c->din_pad; a.h_pad = c->h_pad; a.dout_pad = round_up(c->d, 8);
+    a.norm = c->norm64;
+}
+
 void fill_model_args(ss_ctx* c, RolloutArgs& a) {
     for (int l = 0; l <= c->L; ++l) {
         a.w[l] = c->w32[l].as<float>();
@@ -111,6 +139,8 @@ extern "C" int ss_mpc_set_model(ss_ctx* c, int d, int da, int num_fc_layers, int
     c->h_pad = round_up(depth, 16);
     c->w32.resize(num_fc_layers + 1);
     c->b32.resize(num_fc_layers + 1);
+    c->w64.resize(num_fc_layers + 1);
+    c->b64.resize(num_fc_layers + 1);
     c->hw.assign(num_fc_layers + 1, {});
     c->hb.assign(num_fc_layers + 1, {});
     for (int l = 0; l <= num_fc_layers; ++l) {
@@ -128,6 +158,16 @@ extern "C" int ss_mpc_set_model(ss_ctx* c, int d, int da, int num_fc_layers, int
         SS_CUDA_CHECK(c, cudaMemcpyAsync(c->w32[l].p, w.data(), w.size() * 4, cudaMemcpyHostToDevice, c->stream));
         SS_CUDA_CHECK(c, cudaMemcpyAsync(c->b32[l].p, b.data(), b.size() * 4, cudaMemcpyHostToDevice, c->stream));
         SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));   // w, b are stack-local staging
+        // the caller's doubles as they are for SS_PRECISION_FP64
+        std::vector<double> w64((size_t)in_pad * out_pad, 0.0), b64(out_pad, 0.0);
+        for (int i = 0; i < in; ++i)
+            for (int o = 0; o < out; ++o) w64[(size_t)i * out_pad + o] = weights[l][(size_t)i * out + o];
+        for (int o = 0; o < out; ++o) b64[o] = biases[l][o];
+        SS_CUDA_CHECK(c, c->w64[l].ensure(w64.size() * 8));
+        SS_CUDA_CHECK(c, c->b64[l].ensure(b64.size() * 8));
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->w64[l].p, w64.data(), w64.size() * 8, cudaMemcpyHostToDevice, c->stream));
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->b64[l].p, b64.data(), b64.size() * 8, cudaMemcpyHostToDevice, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
     }
     // Q4 (SURVEY 8a): the reference evaluates nan_to_num((x - mean) / std); for std == 0 that is 0
     // when x == mean and +-1.8e308 otherwise.  A zero-variance feature carries no information, so
@@ -142,6 +182,17 @@ extern "C" int ss_mpc_set_model(ss_ctx* c, int d, int da, int num_fc_layers, int
     for (int j = 0; j < da; ++j) {
         c->norm.mean_y[j] = (float)mean_y[j];
         c->norm.inv_std_y[j] = std_y[j] != 0.0 ? (float)(1.0 / std_y[j]) : 0.f;
+    }
+    std::memset(&c->norm64, 0, sizeof(c->norm64));
+    for (int j = 0; j < d; ++j) {
+        c->norm64.mean_x[j] = mean_x[j];
+        c->norm64.std_x[j] = std_x[j];
+        c->norm64.mean_z[j] = mean_z[j];
+        c->norm64.std_z[j] = std_z[j];
+    }
+    for (int j = 0; j < da; ++j) {
+        c->norm64.mean_y[j] = mean_y[j];
+        c->norm64.std_y[j] = std_y[j];
     }
     c->model_set = true;
     c->run.valid = false;
@@ -175,6 +226,12 @@ extern "C" int ss_mpc_set_plan(ss_ctx* c, const double* desired_states, int W,
     SS_CUDA_CHECK(c, cudaMemcpyAsync(c->plan_dl.p, dl.data(), dl.size() * 4, cudaMemcpyHostToDevice, c->stream));
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
     for (int j = 0; j < SS_MAX_D; ++j) c->inv_radii[j] = j < d ? (float)(1.0 / radii[j]) : 0.f;
+    SS_CUDA_CHECK(c, c->plan_ds64.ensure((size_t)W * d * 8));
+    SS_CUDA_CHECK(c, c->plan_dl64.ensure((size_t)W * 8));
+    SS_CUDA_CHECK(c, cudaMemcpyAsync(c->plan_ds64.p, desired_states, (size_t)W * d * 8, cudaMemcpyHostToDevice, c->stream));
+    SS_CUDA_CHECK(c, cudaMemcpyAsync(c->plan_dl64.p, distances_left, (size_t)W * 8, cudaMemcpyHostToDevice, c->stream));
+    SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+    for (int j = 0; j < SS_MAX_D; ++j) c->radii64[j] = j < d ? radii[j] : 1.0;
     c->W = W;
     c->plan_set = true;
     c->run.valid = false;
@@ -202,6 +259,47 @@ extern "C" int ss_mpc_sample_actions(ss_ctx* c, int64_t K_local, int64_t k_offse
     return SS_OK;
 }
 
+static int reduce_projection_sums(ss_ctx* c, long long n_qcols);
+
+// SS_PRECISION_FP64 rollout of the batch described by c->run (its actions already in place)
+static int rollout_fp64(ss_ctx* c, bool ref) {
+    auto& r = c->run;
+    const int T = r.H + 1, d = c->d;
+    if (c->gpow64_gamma != r.gamma || c->gpow64_T != T || !c->mpc_misc64.p) {
+        std::vector<double> gp(T);
+        for (int t = 0; t < T; ++t) gp[t] = std::pow(r.gamma, (double)t);     // gamma ** t (NND_MB_agent.py:611)
+        // [gamma^t (T, padded to even) | replay rows T x (d + 1)]
+        SS_CUDA_CHECK(c, c->mpc_misc64.ensure(((size_t)T + 2 + (size_t)T * (SS_MAX_D + 1)) * 8));
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->mpc_misc64.p, gp.data(), T * 8, cudaMemcpyHostToDevice, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+        c->gpow64_gamma = r.gamma;
+        c->gpow64_T = T;
+    }
+    Rollout64Args a;
+    std::memset(&a, 0, sizeof(a));
+    fill_model64_args(c, a);
+    a.act = r.act;
+    a.plan = make_plan64(c, r.gamma, r.hpf);
+    for (int j = 0; j < SS_MAX_D; ++j) a.state0[j] = r.state64[j];
+    a.wp_index = r.wp_index; a.H = r.H; a.K_local = r.K_local; a.k_offset = r.k_offset;
+    a.per_sample = !ref;
+    SS_CUDA_CHECK(c, c->mpc_states64.ensure((size_t)T * r.K_local * (d + 1) * 8));
+    SS_CUDA_CHECK(c, c->mpc_scores64.ensure((size_t)r.K_local * 8));
+    a.rows_out = c->mpc_states64.as<double>();
+    a.scores_out = ref ? nullptr : c->mpc_scores64.as<double>();
+    if (ref) {
+        const size_t cols = (size_t)mpc_fp64_grid(r.K_local);
+        SS_CUDA_CHECK(c, c->mpc_partial_sums.ensure((cols + 64) * T * 2 * 8));
+        SS_CUDA_CHECK(c, c->mpc_sums.ensure((size_t)T * 2 * 8));
+        a.qsums = c->mpc_partial_sums.as<double>();
+    }
+    timer_mark(c, "mpc_setup");
+    int rc = mpc_fp64_launch(c, a);
+    if (rc) return rc;
+    r.kernel = 4;
+    return SS_OK;
+}
+
 extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int64_t K_local,
                               int64_t k_offset, int64_t K_global, int H, const double* actions,
                               uint64_t seed, const double* act_low, const double* act_high,
@@ -218,7 +316,7 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
     if (precision == SS_PRECISION_AUTO) precision = c->tc_ready ? SS_PRECISION_BF16_TC : SS_PRECISION_FP32;
     if (precision == SS_PRECISION_BF16_TC && !c->tc_ready)
         SS_FAIL(c, SS_EUNSUPPORTED, "mpc: this model shape has no tcgen05 kernel (use precision FP32 or AUTO)");
-    if (precision != SS_PRECISION_FP32 && precision != SS_PRECISION_BF16_TC)
+    if (precision != SS_PRECISION_FP32 && precision != SS_PRECISION_BF16_TC && precision != SS_PRECISION_FP64)
         SS_FAIL(c, SS_EINVAL, "mpc: unknown precision");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     timer_begin(c);
@@ -230,6 +328,7 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
     r.wp_index = wp_index; r.penalty_mode = penalty_mode; r.precision = precision;
     r.gamma = gamma; r.hpf = hpf;
     for (int j = 0; j < SS_MAX_D; ++j) r.state[j] = j < c->d ? (float)state[j] : 0.f;
+    for (int j = 0; j < SS_MAX_D; ++j) r.state64[j] = j < c->d ? state[j] : 0.0;
     int rc = fill_action_source(c, r.act, H, c->da, seed, act_low, act_high);
     if (rc) return rc;
     const int T = H + 1;
@@ -298,6 +397,13 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
         c->gpow_T = T;
     }
     const float* gpow = c->mpc_replay.as<float>();
+    const bool ref = penalty_mode == SS_PENALTY_REFERENCE;
+    r.states_stored = true;
+    if (precision == SS_PRECISION_FP64) {
+        rc = rollout_fp64(c, ref);
+        if (rc) return rc;
+        return reduce_projection_sums(c, mpc_fp64_grid(K_local));
+    }
 
     RolloutArgs a;
     std::memset(&a, 0, sizeof(a));
@@ -309,11 +415,9 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
     a.per_sample = penalty_mode == SS_PENALTY_PER_SAMPLE;
     SS_CUDA_CHECK(c, c->mpc_scores.ensure((size_t)K_local * 4));
     a.scores_out = c->mpc_scores.as<float>();
-    const bool ref = penalty_mode == SS_PENALTY_REFERENCE;
     // The trajectory rows (state, waypoint index) are spilled in both penalty modes: the stores
     // hide behind the layer-2 MMAs (no measurable cost), the reference-mode passes need them, and the
     // winner's predicted path (NND_MB_agent.py:517) is then a gather instead of a re-roll.
-    r.states_stored = true;
     SS_CUDA_CHECK(c, c->mpc_states.ensure((size_t)T * K_local * traj_row_stride(c->d) * 4));
     a.states_out = c->mpc_states.as<float>();
     // projection sums come out of the rollout kernel: one table column per (tile, row warp) of the tcgen05
@@ -356,12 +460,20 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
         if (rc) return rc;
         r.kernel = mpc_simt_is_thread_kernel(a) ? 3 : 0;
     }
+    return reduce_projection_sums(c, tc_qcols);
+}
+
+// reference penalty: the rollout kernel's [2T][n_qcols] projection-sum columns -> the 2T sums of the batch
+static int reduce_projection_sums(ss_ctx* c, long long n_qcols) {
+    auto& r = c->run;
+    const int T = r.H + 1;
+    int rc = SS_OK;
     timer_mark(c, "mpc_rollout");
     r.sum_cols = nullptr;
     r.n_cols = 0;
     r.sums_reduced = false;
-    if (ref) {
-        int red_blocks = (int)tc_qcols;
+    if (r.penalty_mode == SS_PENALTY_REFERENCE) {
+        int red_blocks = (int)n_qcols;
         const double* red_src = c->mpc_partial_sums.as<double>();
         if (red_blocks > 256) {
             // thousands of columns (one per tile and row warp): fold them to 16 per output first
@@ -374,7 +486,7 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
         // open peer exchange the reduction kernel also all-reduces them over NVLink peer memory (no
         // NCCL call, no host round trip); otherwise the caller all-reduces the buffer
         // ss_mpc_projection_sums returns.
-        r.peer_sums = c->peer_ready && K_global != K_local;
+        r.peer_sums = c->peer_ready && r.K_global != r.K_local;
         rc = r.peer_sums ? peer_allreduce_sums(c, red_src, red_blocks, T, c->mpc_sums.as<double>())
                          : mpc_reduce_sums(c, red_src, red_blocks, T, c->mpc_sums.as<double>());
         if (rc) return rc;
@@ -427,6 +539,16 @@ static int finish_device(ss_ctx* c, int want_path, double* pkg_dst, double* host
         SS_CUDA_CHECK(c, cudaMemsetAsync(c->mpc_result.p, 0, sizeof(MpcResult), c->stream));
     }
     double* bv = c->mpc_block_best.as<double>();
+    if (r.precision == SS_PRECISION_FP64) {
+        int rc = mpc_tail64(c, make_plan64(c, r.gamma, r.hpf), r.wp_index, c->mpc_states64.as<double>(), r.K_local, T,
+                            penalties ? r.sum_cols : nullptr, c->mpc_scores64.as<double>(), r.k_offset, bv,
+                            reinterpret_cast<long long*>(bv + blocks), c->mpc_result.p, r.act, want_path, pkg_dst,
+                            host_pkg, seq);
+        if (rc) return rc;
+        r.finished = true;
+        timer_mark(c, "mpc_tail");
+        return SS_OK;
+    }
     int rc = mpc_tail(c, p, c->mpc_states.as<float>(), r.K_local, T, penalties ? r.sum_cols : nullptr, r.n_cols,
                       c->mpc_scores.as<float>(), r.k_offset, bv, reinterpret_cast<long long*>(bv + blocks),
                       c->mpc_result.p, r.act, want_path, pkg_dst, host_pkg, seq,
@@ -438,6 +560,22 @@ static int finish_device(ss_ctx* c, int want_path, double* pkg_dst, double* host
 }
 
 static int package_count(ss_ctx* c) { return 2 + c->run.H * c->da + (c->run.H + 1) * c->d; }
+
+// the scores of the last finished decision, queued on the stream; widen_scores() completes them after the
+// synchronisation (FP32 buffer widened on the host, float64 buffer copied as it is)
+static int queue_scores(ss_ctx* c, std::vector<float>& sc, double* out_scores) {
+    auto& r = c->run;
+    if (r.precision == SS_PRECISION_FP64) {
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(out_scores, c->mpc_scores64.p, (size_t)r.K_local * 8, cudaMemcpyDeviceToHost, c->stream));
+        return SS_OK;
+    }
+    sc.resize(r.K_local);
+    SS_CUDA_CHECK(c, cudaMemcpyAsync(sc.data(), c->mpc_scores.p, (size_t)r.K_local * 4, cudaMemcpyDeviceToHost, c->stream));
+    return SS_OK;
+}
+static void widen_scores(const std::vector<float>& sc, double* out_scores) {
+    for (size_t k = 0; k < sc.size(); ++k) out_scores[k] = (double)sc[k];
+}
 
 extern "C" int ss_mpc_finish(ss_ctx* c, int64_t* out_best_k, double* out_best_score, double* out_scores) {
     if (!c) return SS_EINVAL;
@@ -451,12 +589,11 @@ extern "C" int ss_mpc_finish(ss_ctx* c, int64_t* out_best_k, double* out_best_sc
     SS_CUDA_CHECK(c, cudaMemcpyAsync(&h, c->mpc_result.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
     std::vector<float> sc;
     if (out_scores) {
-        sc.resize(r.K_local);
-        SS_CUDA_CHECK(c, cudaMemcpyAsync(sc.data(), c->mpc_scores.p, (size_t)r.K_local * 4, cudaMemcpyDeviceToHost, c->stream));
+        rc = queue_scores(c, sc, out_scores);
+        if (rc) return rc;
     }
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
-    if (out_scores)
-        for (int64_t k = 0; k < r.K_local; ++k) out_scores[k] = (double)sc[k];
+    if (out_scores) widen_scores(sc, out_scores);
     if (out_best_k) *out_best_k = h.best_k;
     if (out_best_score) *out_best_score = h.best_score;
     return SS_OK;
@@ -525,6 +662,12 @@ extern "C" int ss_mpc_get_states(ss_ctx* c, double* out_states) {
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     const size_t rows = (size_t)(r.H + 1) * r.K_local;
     const int d = c->d, rs = traj_row_stride(d);
+    if (r.precision == SS_PRECISION_FP64) {
+        SS_CUDA_CHECK(c, cudaMemcpy2DAsync(out_states, d * 8, c->mpc_states64.p, rs * 8, d * 8, rows,
+                                           cudaMemcpyDeviceToHost, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+        return SS_OK;
+    }
     std::vector<float> tmp(rows * rs);
     SS_CUDA_CHECK(c, cudaMemcpyAsync(tmp.data(), c->mpc_states.p, tmp.size() * 4, cudaMemcpyDeviceToHost, c->stream));
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
@@ -556,6 +699,37 @@ static int reroll_winner(ss_ctx* c, int64_t k_global, float* rows_dev) {
     return r.precision == SS_PRECISION_BF16_TC ? mpc_tc_launch(c, a, nullptr) : mpc_simt_launch(c, a, nullptr);
 }
 
+// SS_PRECISION_FP64: the winner's path from the float64 rows (resident, or re-rolled through the fp64 kernel)
+static int replay_path_fp64(ss_ctx* c, int64_t k_global, double* out_path) {
+    auto& r = c->run;
+    const int T = r.H + 1, d = c->d;
+    const int64_t k_local = k_global - r.k_offset;
+    const bool mine = k_local >= 0 && k_local < r.K_local;
+    const double* rows = c->mpc_states64.as<double>() + (size_t)k_local * (d + 1);
+    size_t pitch = (size_t)r.K_local * (d + 1) * 8;
+    if (!(r.states_stored && mine)) {
+        if (r.act.host_actions && !mine)
+            SS_FAIL(c, SS_EINVAL, "mpc: host-provided actions of another shard cannot be replayed here");
+        Rollout64Args a;
+        std::memset(&a, 0, sizeof(a));
+        fill_model64_args(c, a);
+        a.act = r.act;
+        if (a.act.host_actions) a.act.host_actions += (size_t)k_local * r.H * c->da;
+        a.plan = make_plan64(c, r.gamma, r.hpf);
+        for (int j = 0; j < SS_MAX_D; ++j) a.state0[j] = r.state64[j];
+        a.wp_index = r.wp_index; a.H = r.H; a.K_local = 1; a.k_offset = k_global;
+        a.per_sample = 1;
+        a.rows_out = misc64_rows(c);
+        int rc = mpc_fp64_launch(c, a);
+        if (rc) return rc;
+        rows = a.rows_out;
+        pitch = (size_t)(d + 1) * 8;
+    }
+    if (out_path)
+        SS_CUDA_CHECK(c, cudaMemcpy2DAsync(out_path, d * 8, rows, pitch, d * 8, T, cudaMemcpyDeviceToHost, c->stream));
+    return SS_OK;
+}
+
 extern "C" int ss_mpc_replay(ss_ctx* c, int64_t k_global, double* out_sequence, double* out_path) {
     if (!c) return SS_EINVAL;
     auto& r = c->run;
@@ -565,10 +739,14 @@ extern "C" int ss_mpc_replay(ss_ctx* c, int64_t k_global, double* out_sequence, 
     const int T = r.H + 1, d = c->d, da = c->da;
     const int64_t k_local = k_global - r.k_offset;
     const bool mine = k_local >= 0 && k_local < r.K_local;
+    const bool f64 = r.precision == SS_PRECISION_FP64;
     float* rows_dev = c->mpc_replay.as<float>() + (T + SS_MAX_D + 3) / 4 * 4;   // 16-byte aligned rows
     float* path_dev = rows_dev + (size_t)T * (SS_MAX_D + 1);
     int rc = SS_OK;
-    if (r.states_stored && mine) {
+    if (f64) {
+        rc = replay_path_fp64(c, k_global, out_path);
+        if (rc) return rc;
+    } else if (r.states_stored && mine) {
         // the trajectories of this batch are still resident (reference mode): just gather the row
         gather_path_kernel<<<(T * d + 127) / 128, 128, 0, c->stream>>>(c->mpc_states.as<float>(), r.K_local,
                                                                        k_local, T, d, path_dev);
@@ -581,8 +759,8 @@ extern "C" int ss_mpc_replay(ss_ctx* c, int64_t k_global, double* out_sequence, 
         c->launches++;
         SS_CUDA_CHECK(c, cudaGetLastError());
     }
-    std::vector<float> path((size_t)T * d);
-    SS_CUDA_CHECK(c, cudaMemcpyAsync(path.data(), path_dev, path.size() * 4, cudaMemcpyDeviceToHost, c->stream));
+    std::vector<float> path(f64 ? 0 : (size_t)T * d);
+    if (!f64) SS_CUDA_CHECK(c, cudaMemcpyAsync(path.data(), path_dev, path.size() * 4, cudaMemcpyDeviceToHost, c->stream));
     if (out_sequence) {
         const size_t n = (size_t)r.H * da;
         SS_CUDA_CHECK(c, c->mpc_block_best.ensure(1024 * 16 + n * 8));
@@ -595,7 +773,7 @@ extern "C" int ss_mpc_replay(ss_ctx* c, int64_t k_global, double* out_sequence, 
         SS_CUDA_CHECK(c, cudaMemcpyAsync(out_sequence, seq_dev, n * 8, cudaMemcpyDeviceToHost, c->stream));
     }
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
-    if (out_path)
+    if (out_path && !f64)
         for (size_t i = 0; i < path.size(); ++i) out_path[i] = (double)path[i];
     timer_mark(c, "mpc_replay");
     return SS_OK;
@@ -622,13 +800,17 @@ extern "C" int ss_mpc_plan(ss_ctx* c, const double* state, int wp_index, int64_t
     std::vector<double> pkg(n);
     std::vector<float> sc;
     if (out_scores) {
-        sc.resize(K_local);
-        SS_CUDA_CHECK(c, cudaMemcpyAsync(sc.data(), c->mpc_scores.p, (size_t)K_local * 4, cudaMemcpyDeviceToHost, c->stream));
+        rc = queue_scores(c, sc, out_scores);
+        if (rc) return rc;
     }
     rc = ss_mpc_read_package(c, pkg.data(), n);       // the one host synchronisation of the decision
     if (rc) return rc;
-    if (out_scores)
-        for (int64_t k = 0; k < K_local; ++k) out_scores[k] = (double)sc[k];
+    if (out_scores) {
+        // the package may have come through mapped host memory without a stream synchronisation, and the
+        // float64 scores were copied straight into the caller's array (which may be pinned)
+        if (c->run.precision == SS_PRECISION_FP64) SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+        widen_scores(sc, out_scores);
+    }
     if (out_best_score) *out_best_score = pkg[0];
     if (out_best_k) *out_best_k = (int64_t)pkg[1];
     const int n_seq = H * c->da;

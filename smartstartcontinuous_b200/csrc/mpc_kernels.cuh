@@ -27,6 +27,35 @@ struct RolloutArgs {
                              // 32 rows of every (tile, row warp), or null (per-sample penalty)
 };
 
+// float64 rollout (mpc_fp64.cu): every operand and every operation in float64, the reference's element-wise
+// operation order (score.cuh, float64 twin)
+struct Rollout64Args {
+    const double* w[SS_MAX_LAYERS + 1];     // [in_pad_l][out_pad_l], zero padded like RolloutArgs
+    const double* b[SS_MAX_LAYERS + 1];
+    int d, da, L, h;
+    int din_pad, h_pad, dout_pad;
+    MpcNorm64 norm;
+    ActionSource act;
+    Plan64 plan;
+    double state0[SS_MAX_D];
+    int wp_index, H;
+    long long K_local, k_offset;
+    int per_sample;          // 1: final scores (per-sample penalty); 0: reference mode, the tail scores the rows
+    double* rows_out;        // [H+1][K_local][d + 1] (state, waypoint index after the move)
+    double* scores_out;      // [K_local] (per-sample mode) or null
+    double* qsums;           // reference mode: [H+1][2][ceil(K_local / 32)] a'.b' and b'.b' per 32 sequences, or null
+};
+int mpc_fp64_launch(ss_ctx* c, const Rollout64Args& a);
+int mpc_fp64_grid(long long K_local);      // = projection-sum columns
+size_t mpc_fp64_smem_bytes(int din_pad, int h_pad);
+int mpc_fp64_widen(ss_ctx* c, const float* W, const float* b, int in, int out, int out_pad, double* Wp, double* bp);
+// float64 tail: penalties (reference mode: every score recomputed from the rows in the reference's order),
+// arg-max and package, like mpc_tail
+int mpc_tail64(ss_ctx* c, const Plan64& plan, int wp_index, const double* rows, long long K_local, int T,
+               const double* sums, double* scores, long long k_offset, double* block_v, long long* block_i,
+               void* result_dev, const ActionSource& act, int want_path, double* pkg, double* host_pkg,
+               unsigned long long seq);
+
 // fp32 SIMT rollout (mpc_simt.cu)
 int mpc_simt_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out);
 int mpc_simt_grid(const RolloutArgs& a);

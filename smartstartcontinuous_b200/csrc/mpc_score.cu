@@ -61,11 +61,11 @@ struct TailOut {
     float* scores_final;            // where the final scores go (== scores in place)
 };
 
-// the winner's package: [score, k (global), sequence (H*da), path (T*d)] -- kept out of line so that its
-// Philox / float64 code does not inflate the register count of the bandwidth-bound penalty loop
-__device__ __noinline__ void tail_write_package(double best_v, long long kl, long long k_offset, const float* rows,
-                                                long long K, int T, int d, const ActionSource* actp, int want_path,
-                                                TailOut out) {
+// the winner's package: [score, k (global), sequence (H*da), path (T*d)]; rows of d + 1 values (state, waypoint index)
+template <typename Row>
+__device__ __forceinline__ void write_package(double best_v, long long kl, long long k_offset, const Row* rows,
+                                              long long K, int T, int d, const ActionSource* actp, int want_path,
+                                              TailOut out) {
     const ActionSource& act = *actp;
     const int tid = threadIdx.x;
     const long long kg = kl < 0 ? -1 : kl + k_offset;
@@ -87,6 +87,19 @@ __device__ __noinline__ void tail_write_package(double best_v, long long kl, lon
         out.pkg[o] = val;
         if (hp) host_slot_put(hp, o, val, tag);      // self-validating: no fence, barrier or flag behind it
     }
+}
+
+// kept out of line so that its Philox / float64 code does not inflate the register count of the
+// bandwidth-bound penalty loop
+__device__ __noinline__ void tail_write_package(double best_v, long long kl, long long k_offset, const float* rows,
+                                                long long K, int T, int d, const ActionSource* actp, int want_path,
+                                                TailOut out) {
+    write_package<float>(best_v, kl, k_offset, rows, K, T, d, actp, want_path, out);
+}
+__device__ __noinline__ void tail_write_package(double best_v, long long kl, long long k_offset, const double* rows,
+                                                long long K, int T, int d, const ActionSource* actp, int want_path,
+                                                TailOut out) {
+    write_package<double>(best_v, kl, k_offset, rows, K, T, d, actp, want_path, out);
 }
 
 template <int DT>
@@ -172,6 +185,86 @@ mpc_tail_kernel(const PlanView Pg, const float* __restrict__ rows, long long K, 
     tail_write_package(s_v[0], s_i[0], k_offset, rows, K, T, Pg.d, &act, want_path, out);
 }
 
+// float64 tail (SS_PRECISION_FP64), one sequence per thread.  Reference penalty (sums != null): the score is
+// recomputed from the rows in the reference's order -- per step the progress term, then the penalty with the
+// step's global coefficient lambda_t = sum a'.b' / sum b'.b' (float64) -- so it is the reference's sum, not the
+// progress sum minus the penalty sum.  Per-sample penalty: the rollout kernel's scores are final.
+template <int DT>
+__global__ void __launch_bounds__(128)
+mpc_tail64_kernel(const Plan64 P, int wp_index, const double* __restrict__ rows, long long K, int T,
+                  const double* __restrict__ sums, double* __restrict__ scores, long long k_offset,
+                  double* __restrict__ block_v, long long* __restrict__ block_i, MpcResult* __restrict__ result,
+                  ActionSource act, int want_path, TailOut out) {
+    extern __shared__ double s_lam64[];          // [T]
+    pdl_wait();
+    __shared__ double s_v[32];
+    __shared__ long long s_i[32];
+    __shared__ bool s_last;
+    const int tid = threadIdx.x;
+    const long long k = blockIdx.x * (long long)blockDim.x + tid;
+    if (sums) {
+        for (int t = tid; t < T; t += blockDim.x) s_lam64[t] = sums[2 * t] / sums[2 * t + 1];
+        __syncthreads();
+    }
+    double v = 0.0;
+    long long bi = -1;
+    if (k < K) {
+        double score;
+        if (sums) {
+            const int d = P.d;
+            double x[DT];
+            ScoreAcc64 sc;
+            for (int t = 0; t < T; ++t) {
+                const double* row = rows + ((size_t)t * K + k) * (d + 1);
+#pragma unroll
+                for (int j = 0; j < DT; ++j) x[j] = j < d ? __ldg(row + j) : 0.0;
+                const int idx = (int)__ldg(row + d);
+                if (t == 0) score_init64<DT>(P, wp_index, x, sc);
+                // to_end = distances_left[idx] + dist(desired_states[idx], x) with idx after the move (dc after
+                // :605 is dn exactly when the sample moved)
+                const double to_end = P.dl[idx] + ell_dist64<DT>(P, P.ds + (size_t)idx * d, x);
+                sc.score = sc.score + __dmul_rn(sc.prev - to_end, P.gpow[t]);
+                sc.prev = to_end;
+                sc.score = sc.score - penalty64<DT>(P, idx, x, s_lam64[t]);
+            }
+            score = sc.score;
+            scores[k] = score;
+        } else {
+            score = scores[k];
+        }
+        v = score;
+        bi = k;
+    }
+    // (the arg-max / package part of mpc_tail_kernel; kept as a copy so that the FP32 tail's code stays as it was)
+    block_argmax(v, bi, s_v, s_i);
+    if (tid == 0) {
+        block_v[blockIdx.x] = v;
+        block_i[blockIdx.x] = bi;
+        __threadfence();
+        s_last = atomicAdd(&result->blocks_done, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    v = 0.0;
+    bi = -1;
+    for (int b = tid; b < gridDim.x; b += blockDim.x) {
+        const double ov = __ldcg(block_v + b);
+        const long long oi = __ldcg(block_i + b);
+        if (argmax_better(ov, oi, v, bi)) { v = ov; bi = oi; }
+    }
+    block_argmax(v, bi, s_v, s_i);
+    if (tid == 0) {
+        s_v[0] = v;
+        s_i[0] = bi;
+        result->best_score = v;
+        result->best_k = bi < 0 ? -1 : bi + k_offset;
+        result->blocks_done = 0;
+    }
+    __syncthreads();
+    tail_write_package(s_v[0], s_i[0], k_offset, rows, K, T, P.d, &act, want_path, out);
+}
+
 }  // namespace
 
 int mpc_reduce_sums(ss_ctx* c, const double* partial, int blocks, int T, double* sums) {
@@ -223,6 +316,29 @@ int mpc_tail(ss_ctx* c, const PlanView& plan, const float* rows, long long K_loc
     else if (plan.d <= 8) TAIL_LAUNCH(8);
     else TAIL_LAUNCH(SS_MAX_D);
 #undef TAIL_LAUNCH
+    SS_CUDA_CHECK(c, e);
+    c->launches++;
+    SS_CUDA_CHECK(c, cudaGetLastError());
+    return SS_OK;
+}
+
+int mpc_tail64(ss_ctx* c, const Plan64& plan, int wp_index, const double* rows, long long K_local, int T,
+               const double* sums, double* scores, long long k_offset, double* block_v, long long* block_i,
+               void* result_dev, const ActionSource& act, int want_path, double* pkg, double* host_pkg,
+               unsigned long long seq) {
+    const dim3 g((unsigned)mpc_tail_blocks(K_local)), b((unsigned)mpc_tail_threads(K_local));
+    const size_t smem = (size_t)T * sizeof(double);
+    TailOut out;
+    out.pkg = pkg; out.host_pkg = host_pkg; out.seq = seq; out.sums_out = nullptr; out.scores_final = nullptr;
+    MpcResult* res = reinterpret_cast<MpcResult*>(result_dev);
+    cudaError_t e;
+#define TAIL64_LAUNCH(DT_)                                                                                         \
+    e = launch_dependent(mpc_tail64_kernel<DT_>, g, b, smem, c->stream, plan, wp_index, rows, K_local, T, sums,   \
+                         scores, k_offset, block_v, block_i, res, act, want_path, out)
+    if (plan.d <= 4) TAIL64_LAUNCH(4);
+    else if (plan.d <= 8) TAIL64_LAUNCH(8);
+    else TAIL64_LAUNCH(SS_MAX_D);
+#undef TAIL64_LAUNCH
     SS_CUDA_CHECK(c, e);
     c->launches++;
     SS_CUDA_CHECK(c, cudaGetLastError());

@@ -161,3 +161,133 @@ __device__ __forceinline__ float penalty_with_lambda(const PlanView& P, int idx_
         }
     return sqrtf(s) * P.pen_scale;
 }
+
+// ---- float64 twin (SS_PRECISION_FP64, mpc_fp64.cu / the float64 tail of mpc_score.cu) ---------------------------
+// The reference's own operation order, element by element: the products are __dmul_rn so that the compiler
+// cannot contract them into an FMA with the following add, divisions divide, and the sums over the state
+// dimension run in numpy's order (pairwise_sum of numpy/core/src/umath/loops_utils.h: plain left-to-right
+// below 8 terms, eight interleaved accumulators above).
+struct Plan64 {
+    const double* ds;        // desired_states [W][d]
+    const double* dl;        // distances_left [W]
+    const double* gpow;      // gamma ** t, t = 0..H  (host pow in float64)
+    int W, d;
+    double r[SS_MAX_D];      // radii
+    double hpf, gamma;
+};
+
+struct ScoreAcc64 {
+    int idx;
+    double prev, score;
+};
+
+template <int DT>
+__device__ __forceinline__ double np_sum(const double (&v)[DT], int n) {
+    if (n < 8) {
+        double s = 0.0;
+#pragma unroll
+        for (int j = 0; j < DT; ++j)
+            if (j < n) s = __dadd_rn(s, v[j]);
+        return s;
+    }
+    double r[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) r[q] = v[q < DT ? q : 0];
+    const int n8 = n - n % 8;
+#pragma unroll
+    for (int j = 8; j < DT; ++j)
+        if (j < n8) r[j % 8] = __dadd_rn(r[j % 8], v[j]);
+    double s = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])),
+                         __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
+#pragma unroll
+    for (int j = 8; j < DT; ++j)
+        if (j >= n8 && j < n) s = __dadd_rn(s, v[j]);
+    return s;
+}
+
+// numerical.py:116-124: sqrt(sum(((a - b) / r) ** 2))
+template <int DT>
+__device__ __forceinline__ double ell_dist64(const Plan64& P, const double* __restrict__ w, const double (&x)[DT]) {
+    double q[DT];
+#pragma unroll
+    for (int j = 0; j < DT; ++j) {
+        q[j] = 0.0;
+        if (j < P.d) {
+            const double df = (w[j] - x[j]) / P.r[j];
+            q[j] = __dmul_rn(df, df);
+        }
+    }
+    return sqrt(np_sum<DT>(q, P.d));
+}
+
+template <int DT>
+__device__ __forceinline__ void score_init64(const Plan64& P, int wp_index, const double (&x0)[DT], ScoreAcc64& a) {
+    a.idx = wp_index;
+    a.prev = P.dl[wp_index] + ell_dist64<DT>(P, P.ds + (size_t)wp_index * P.d, x0);
+    a.score = 0.0;
+}
+
+// a' = (x - w0) / r, b' = (w1 - w0) / r of the segment the point projects on (numerical.py:76-88)
+template <int DT>
+__device__ __forceinline__ void proj_vectors64(const Plan64& P, int idx, const double (&x)[DT], double (&av)[DT],
+                                               double (&bv)[DT]) {
+    const int b0 = idx - 1 > 0 ? idx - 1 : 0;
+    const double* w0 = P.ds + (size_t)b0 * P.d;
+    const double* w1 = w0 + P.d;
+#pragma unroll
+    for (int j = 0; j < DT; ++j) {
+        av[j] = 0.0;
+        bv[j] = 0.0;
+        if (j < P.d) {
+            av[j] = (x[j] - w0[j]) / P.r[j];
+            bv[j] = (w1[j] - w0[j]) / P.r[j];
+        }
+    }
+}
+
+// sum(a' * b') and sum(b' * b') (numerical.py:89-93, per point)
+template <int DT>
+__device__ __forceinline__ void proj_terms64(const Plan64& P, int idx, const double (&x)[DT], double& ab, double& bb) {
+    double av[DT], bv[DT];
+    proj_vectors64<DT>(P, idx, x, av, bv);
+#pragma unroll
+    for (int j = 0; j < DT; ++j) { av[j] = __dmul_rn(av[j], bv[j]); bv[j] = __dmul_rn(bv[j], bv[j]); }
+    ab = np_sum<DT>(av, P.d);
+    bb = np_sum<DT>(bv, P.d);
+}
+
+// pen * hpf * gamma of numerical.py:80-81 / NND_MB_agent.py:622 for a given coefficient lam
+template <int DT>
+__device__ __forceinline__ double penalty64(const Plan64& P, int idx, const double (&x)[DT], double lam) {
+    double av[DT], bv[DT];
+    proj_vectors64<DT>(P, idx, x, av, bv);
+#pragma unroll
+    for (int j = 0; j < DT; ++j) {
+        const double df = __dmul_rn(lam, bv[j]) - av[j];
+        av[j] = __dmul_rn(df, df);
+    }
+    return __dmul_rn(__dmul_rn(sqrt(np_sum<DT>(av, P.d)), P.hpf), P.gamma);
+}
+
+// waypoint move + progress term of one point (NND_MB_agent.py:582-611); returns to_end
+template <int DT>
+__device__ __forceinline__ void progress64(const Plan64& P, int t, const double (&x)[DT], ScoreAcc64& a) {
+    const int last = P.W - 1;
+    const int nxt = a.idx + 1 < last ? a.idx + 1 : last;
+    double dc = ell_dist64<DT>(P, P.ds + (size_t)a.idx * P.d, x);
+    const double dn = ell_dist64<DT>(P, P.ds + (size_t)nxt * P.d, x);
+    const bool mv = ((dc <= 1.0) || (dn <= dc)) && (a.idx != last);
+    if (mv) { a.idx += 1; dc = dn; }
+    const double to_end = P.dl[a.idx] + dc;
+    a.score = a.score + __dmul_rn(a.prev - to_end, P.gpow[t]);
+    a.prev = to_end;
+}
+
+// the whole step with the per-sample coefficient (SS_PENALTY_PER_SAMPLE)
+template <int DT>
+__device__ __forceinline__ void score_point64_per_sample(const Plan64& P, int t, const double (&x)[DT], ScoreAcc64& a) {
+    progress64<DT>(P, t, x, a);
+    double ab, bb;
+    proj_terms64<DT>(P, a.idx, x, ab, bb);
+    a.score = a.score - penalty64<DT>(P, a.idx, x, ab / bb);
+}

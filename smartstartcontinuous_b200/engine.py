@@ -17,13 +17,13 @@ import numpy as np
 
 from . import _lib
 from ._lib import (PENALTY_PER_SAMPLE, PENALTY_REFERENCE, PRECISION_AUTO, PRECISION_BF16_TC,
-                   PRECISION_FP32)
+                   PRECISION_FP32, PRECISION_FP64)
 
 _PENALTY = {"reference": PENALTY_REFERENCE, "per_sample": PENALTY_PER_SAMPLE,
             PENALTY_REFERENCE: PENALTY_REFERENCE, PENALTY_PER_SAMPLE: PENALTY_PER_SAMPLE}
-_PRECISION = {"fp32": PRECISION_FP32, "bf16_tc": PRECISION_BF16_TC, "auto": PRECISION_AUTO,
+_PRECISION = {"fp32": PRECISION_FP32, "bf16_tc": PRECISION_BF16_TC, "auto": PRECISION_AUTO, "fp64": PRECISION_FP64,
               PRECISION_FP32: PRECISION_FP32, PRECISION_BF16_TC: PRECISION_BF16_TC,
-              PRECISION_AUTO: PRECISION_AUTO}
+              PRECISION_AUTO: PRECISION_AUTO, PRECISION_FP64: PRECISION_FP64}
 
 
 def _f64(a):
@@ -433,7 +433,7 @@ class Engine:
     def last_rollout_kernel(self):
         """Name of the rollout kernel the last decision ran on."""
         return {0: "mpc_rollout_simt_kernel", 1: "mpc_rollout_tc_kernel", 2: "mpc_rollout_tc_quad_kernel",
-                3: "mpc_rollout_thread_kernel"}.get(
+                3: "mpc_rollout_thread_kernel", 4: "mpc_rollout_fp64_kernel"}.get(
             int(self._lib.ss_mpc_last_kernel(self._h)))
 
     def set_plan(self, desired_states, distances_left, radii):
@@ -579,7 +579,8 @@ class Engine:
         return out
 
     def forward_sim(self, state, actions, precision="fp32"):
-        """Dyn_Model.do_forward_sim(many_in_parallel=True) on the GPU: [H+1, K, d]."""
+        """Dyn_Model.do_forward_sim(many_in_parallel=True) on the GPU: [H+1, K, d] ("fp64": the reference's
+        float64 arithmetic)."""
         if not getattr(self, "_plan_set", False):
             d = self._model_shape[0]
             self.set_plan(np.stack([np.zeros(d), np.ones(d)]), [1.0, 0.0], np.ones(d))

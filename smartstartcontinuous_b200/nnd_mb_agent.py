@@ -14,7 +14,10 @@ and method names are the reference's.  What changed underneath:
 Extra keyword-only options (all default to the reference behaviour):
   engine / device     share an Engine or create one on cuda:<device>
   penalty_mode        "reference" (global projection coefficient, Q1) | "per_sample"
-  precision           "auto" | "fp32" | "bf16_tc"
+  precision           "auto" | "fp32" | "bf16_tc" | "fp64"; "fp64" rolls out and scores in float64 like the
+                      reference (its decision up to the summation order of the GEMMs and reductions, also
+                      when the best two scores are closer than the FP32 / BF16 tolerances), several times
+                      slower than "bf16_tc"; "auto" never picks it
   device_sampling     False: the actions of numpy.random.uniform exactly like :500-501 -- the global
                       MT19937 stream, generated on the GPU from np.random.get_state() and advanced with
                       set_state (host_rng=True draws them on the host and uploads them instead, False
