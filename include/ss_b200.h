@@ -266,8 +266,9 @@ int ss_mpc_last_kernel(ss_ctx* ctx);
 /* ---- dynamics-model training on the device (SURVEY 8f, row f1) ------------------------------
  * Replaces Dyn_Model.train (dynamics_model.py:52-171) as NND_MB_agent.train_dynamics_model calls it
  * (NND_MB_agent.py:437-480): mini-batch Adam (tf.train.AdamOptimizer defaults) on
- * reduce_mean(square(z - f(x))) for the network set with ss_mpc_set_model.  Data sets, FP32 master
- * parameters and Adam moments stay on the device across calls.
+ * reduce_mean(square(z - f(x))) for the network set with ss_mpc_set_model.  Data sets, master
+ * parameters and Adam moments stay on the device across calls, in FP32 (default) or, after
+ * ss_dyn_set_precision(ctx, SS_PRECISION_FP64), in float64 like the reference's graph.
  *   ss_dyn_set_data       which = 0: the initial ("old") data set, 1: the aggregated ("new") one;
  *                         X [n, d + da] normalised inputs, Z [n, d] normalised state deltas
  *   ss_dyn_train_batches  n_batches Adam steps; batch i = old rows idx_old[i*n_old ..] followed by
@@ -279,7 +280,11 @@ int ss_mpc_last_kernel(ss_ctx* ctx);
  *   ss_dyn_commit         re-pack the trained parameters for the rollout kernels on the device (no
  *                         host round trip); ss_mpc_plan uses them from then on
  *   ss_dyn_get_params     export as float64 [in, out] / [out] (checkpoints, tests)
- *   ss_dyn_reset_optimizer  forget the Adam moments and step count */
+ *   ss_dyn_reset_optimizer  forget the Adam moments and step count
+ * With SS_PRECISION_FP64 the data sets are stored without float32 rounding, every step runs in float64
+ * (DFMA; Adam in the oracle's operation order), ss_dyn_get_params returns the float64 masters exactly
+ * and ss_dyn_commit hands them unchanged to SS_PRECISION_FP64 rollouts (the FP32 and tcgen05 images
+ * are packed from the masters rounded once to float). */
 int ss_dyn_set_data(ss_ctx* ctx, int which, const double* X, const double* Z, int64_t n_rows);
 int ss_dyn_train_batches(ss_ctx* ctx, const int32_t* idx_old, const int32_t* idx_new, int n_batches, int n_old,
                          int n_new, double lr, double* out_losses);
@@ -287,6 +292,12 @@ int ss_dyn_eval_loss(ss_ctx* ctx, int which, int batchsize, double* out_mean_los
 int ss_dyn_commit(ss_ctx* ctx);
 int ss_dyn_get_params(ss_ctx* ctx, double* const* out_weights, double* const* out_biases);
 int ss_dyn_reset_optimizer(ss_ctx* ctx);
+/* precision of the device trainer: SS_PRECISION_FP32 (default, today's trainer) or SS_PRECISION_FP64.
+ * Changing it discards the trainer state -- master parameters, Adam moments, step count and both data
+ * sets -- so the next training call starts from the parameters of the last ss_mpc_set_model, as after
+ * ss_dyn_reset_optimizer; the data sets must be uploaded again.  Setting the current value is a no-op.
+ * Any other value: SS_EINVAL. */
+int ss_dyn_set_precision(ss_ctx* ctx, int precision);
 
 /* ---- critic value batch in front of the UCB (SURVEY 8f, row f4) --------------------------
  * V_j = critic(q_j, actor(q_j)) of the DDPG base agent (agent.get_state_value,

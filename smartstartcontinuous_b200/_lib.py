@@ -91,6 +91,7 @@ SIGNATURES = {
     "ss_dyn_commit": (C.c_int, [C.c_void_p]),
     "ss_dyn_get_params": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     "ss_dyn_reset_optimizer": (C.c_int, [C.c_void_p]),
+    "ss_dyn_set_precision": (C.c_int, [C.c_void_p, C.c_int]),
     "ss_value_net_set": (C.c_int, [C.c_void_p, C.c_void_p]),
     "ss_value_net_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "ss_mirror_write": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_int64, C.c_int64, C.c_void_p]),

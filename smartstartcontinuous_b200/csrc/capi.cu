@@ -68,7 +68,7 @@ extern "C" int ss_destroy(ss_ctx* c) {
                       &c->geom_in, &c->geom_rows, &c->geom_pairs, &c->mirror_s, &c->mirror_s2, &c->mirror_idx, &c->mirror_mom,
                       &c->mirror_stage, &c->value_net_params,
                       &c->tc_b3, &c->dyn_params, &c->dyn_m, &c->dyn_v, &c->dyn_x[0], &c->dyn_x[1], &c->dyn_z[0], &c->dyn_z[1],
-                      &c->dyn_act, &c->dyn_scratch, &c->dyn_idx, &c->dyn_losses,
+                      &c->dyn_act, &c->dyn_scratch, &c->dyn_idx, &c->dyn_losses, &c->dyn_round,
                       &c->plan_ds64, &c->plan_dl64, &c->mpc_states64, &c->mpc_scores64, &c->mpc_misc64};
     for (DevBuf* b : bufs) b->release();
     for (auto& b : c->w32) b.release();

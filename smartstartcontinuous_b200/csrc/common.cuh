@@ -162,9 +162,11 @@ struct ss_ctx {
     std::vector<std::vector<double>> hw, hb;   // host copies of the float64 parameters
     std::vector<DevBuf> w64, b64;      // padded float64 weights / biases (SS_PRECISION_FP64), same layout as w32 / b32
     MpcNorm64 norm64;
-    // ---- dynamics-model training on the device (dyn_train.cu): FP32 master parameters, Adam moments,
-    // both training sets, per-batch activations
+    // ---- dynamics-model training on the device (dyn_train.cu): master parameters, Adam moments, both
+    // training sets, per-batch activations -- float, or double when dyn_fp64 (ss_dyn_set_precision)
     DevBuf dyn_params, dyn_m, dyn_v, dyn_x[2], dyn_z[2], dyn_act, dyn_scratch, dyn_idx, dyn_losses;
+    DevBuf dyn_round;                  // float64 masters rounded to float (ss_dyn_commit after FP64 training)
+    bool dyn_fp64 = false;             // the trainer runs in float64 (SS_PRECISION_FP64)
     int64_t dyn_rows[2] = {0, 0};
     long long dyn_t = 0;               // Adam step counter (persists across training calls like TF's slots)
     bool dyn_adam_valid = false;       // moments / counter belong to the current model shape

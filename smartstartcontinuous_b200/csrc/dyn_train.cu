@@ -7,8 +7,8 @@
 // linear output; tf.train.AdamOptimizer defaults beta1 .9, beta2 .999, eps 1e-8; loss =
 // reduce_mean(square(z - f(x))) over batch x outputs) and feeds numpy batches through sess.run.
 //
-// Here everything stays on the GPU: both data sets (FP32), the FP32 master parameters, the Adam
-// moments and the step counter live in the context; a training epoch uploads only the batch row
+// Here everything stays on the GPU: both data sets, the master parameters, the Adam moments and the
+// step counter live in the context; a training epoch uploads only the batch row
 // indices (drawn on the host with the reference's numpy calls, so the batches are the reference's)
 // and queues, per Adam step, a fixed sequence of kernels:
 //
@@ -31,6 +31,15 @@
 // zero amplify operand noise: already FP32 drifts from the float64 oracle by 7e-4 of the movement
 // (Frobenius) after 40 steps, exactly as a float32 numpy run of the oracle does; BF16/TF32 operands
 // would put 1e-3 relative noise on every gradient (tests/test_gpu_dyn_train.py states the bounds).
+//
+// SS_PRECISION_FP64 (ss_dyn_set_precision): the same kernels instantiated for double -- data sets
+// stored without float32 rounding, float64 masters, moments and activations in the same buffers, DFMA
+// GEMMs (not DMMA: 37.0 vs 36.0 TFLOP/s measured, profiles/r03_fp64_time.json, too close to pay for
+// fragment shuffling), and Adam in the oracle's operation order with every product and sum rounded on
+// its own.  A step then differs from oracle/dyn_train_oracle.py only in the summation order of the GEMMs
+// and of the batch reductions (tests/test_gpu_dyn_train_fp64.py).  ss_dyn_commit hands the float64
+// masters unchanged to the float64 rollout and packs the FP32 / tcgen05 images from them rounded once
+// to float.
 #include <cstring>
 
 #include "mpc_kernels.cuh"
@@ -39,51 +48,80 @@ namespace {
 
 constexpr int DYN_MAX_LAYERS = SS_MAX_LAYERS + 1;
 
+// Every training kernel is a template on the scalar type T: float (the FP32 trainer) or double
+// (SS_PRECISION_FP64: masters, moments, data and activations in float64, DFMA).  The helpers below map
+// to fmaf / fmaxf for float, so the FP32 trainer's instructions do not depend on the templating.
+__device__ __forceinline__ float fma_t(float a, float b, float c) { return fmaf(a, b, c); }
+__device__ __forceinline__ double fma_t(double a, double b, double c) { return fma(a, b, c); }
+__device__ __forceinline__ float relu_t(float a) { return fmaxf(a, 0.f); }
+__device__ __forceinline__ double relu_t(double a) { return fmax(a, 0.0); }
+
+template <typename T>
 struct AdamArgs {
-    float lr_t;        // lr * sqrt(1 - beta2^t) / (1 - beta1^t)   (tf.train.AdamOptimizer)
-    float beta1, beta2, eps;
-    float omb1, omb2;  // 1 - beta, rounded once from float64 (1.f - 0.999f is off by 1e-5 relative)
+    T lr_t;            // lr * sqrt(1 - beta2^t) / (1 - beta1^t)   (tf.train.AdamOptimizer)
+    T beta1, beta2, eps;
+    T omb1, omb2;      // 1 - beta, rounded once from float64 (1.f - 0.999f is off by 1e-5 relative)
 };
 
-__device__ __forceinline__ void adam_update(float g, float& w, float& m, float& v, const AdamArgs& a) {
+__device__ __forceinline__ void adam_update(float g, float& w, float& m, float& v, const AdamArgs<float>& a) {
     m = a.beta1 * m + a.omb1 * g;
     v = a.beta2 * v + a.omb2 * g * g;
     w -= a.lr_t * m / (sqrtf(v) + a.eps);
 }
+// float64: oracle/dyn_train_oracle.adam_step operation for operation (m *= b1; m += (1 - b1) g;
+// v *= b2; v += (1 - b2) g g; w -= lr_t m / (sqrt(v) + eps)), every product and sum rounded on its own
+// (no FMA contraction), so a step differs from the oracle only through the gradient's summation order
+__device__ __forceinline__ void adam_update(double g, double& w, double& m, double& v, const AdamArgs<double>& a) {
+    m = __dadd_rn(__dmul_rn(a.beta1, m), __dmul_rn(a.omb1, g));
+    v = __dadd_rn(__dmul_rn(a.beta2, v), __dmul_rn(__dmul_rn(a.omb2, g), g));
+    w = __dsub_rn(w, __ddiv_rn(__dmul_rn(a.lr_t, m), __dadd_rn(__dsqrt_rn(v), a.eps)));
+}
+
+// dynamic shared memory of the first-layer kernel, typed per instantiation
+template <typename T> __device__ __forceinline__ T* dyn_smem();
+template <> __device__ __forceinline__ float* dyn_smem<float>() {
+    extern __shared__ float s_x[];
+    return s_x;
+}
+template <> __device__ __forceinline__ double* dyn_smem<double>() {
+    extern __shared__ double s_x64[];
+    return s_x64;
+}
 
 // ---- forward, first layer: gather + Linear + ReLU ---------------------------------------------
 // batch row b < n_old: old data row idx_old[b]; else new data row idx_new[b - n_old]
+template <typename T>
 __global__ void __launch_bounds__(256)
-dyn_first_layer_kernel(const float* __restrict__ x_old, const float* __restrict__ z_old,
-                       const float* __restrict__ x_new, const float* __restrict__ z_new,
+dyn_first_layer_kernel(const T* __restrict__ x_old, const T* __restrict__ z_old,
+                       const T* __restrict__ x_new, const T* __restrict__ z_new,
                        const int* __restrict__ idx_old, const int* __restrict__ idx_new, int n_old, int B, int din,
-                       int dout, const float* __restrict__ W0, const float* __restrict__ b0, int h, int relu,
-                       float* __restrict__ X, float* __restrict__ Z, float* __restrict__ H1) {
-    extern __shared__ float s_x[];          // [rows_per_block][din]
+                       int dout, const T* __restrict__ W0, const T* __restrict__ b0, int h, int relu,
+                       T* __restrict__ X, T* __restrict__ Z, T* __restrict__ H1) {
+    T* s_x = dyn_smem<T>();                 // [rows_per_block][din]
     const int rows = blockDim.x / 32;       // one warp per batch row
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * rows + warp;
     if (b >= B) return;
     const bool is_old = b < n_old;
     const long long r = is_old ? idx_old[b] : idx_new[b - n_old];
-    const float* xs = (is_old ? x_old : x_new) + (size_t)r * din;
-    const float* zs = (is_old ? z_old : z_new) + (size_t)r * dout;
-    float* sx = s_x + warp * din;
+    const T* xs = (is_old ? x_old : x_new) + (size_t)r * din;
+    const T* zs = (is_old ? z_old : z_new) + (size_t)r * dout;
+    T* sx = s_x + warp * din;
     for (int j = lane; j < din; j += 32) {
-        const float v = xs[j];
+        const T v = xs[j];
         sx[j] = v;
         X[(size_t)b * din + j] = v;
     }
     for (int j = lane; j < dout; j += 32) Z[(size_t)b * dout + j] = zs[j];
     __syncwarp();
     for (int n = lane; n < h; n += 32) {
-        float acc = b0[n];
-        for (int j = 0; j < din; ++j) acc = fmaf(sx[j], W0[(size_t)j * h + n], acc);
-        H1[(size_t)b * h + n] = relu ? fmaxf(acc, 0.f) : acc;
+        T acc = b0[n];
+        for (int j = 0; j < din; ++j) acc = fma_t(sx[j], W0[(size_t)j * h + n], acc);
+        H1[(size_t)b * h + n] = relu ? relu_t(acc) : acc;
     }
 }
 
-// ---- tiled FP32 GEMM: C[i][j] = sum_p A(i, p) * B(p, j) ------------------------------------------
+// ---- tiled GEMM: C[i][j] = sum_p A(i, p) * B(p, j) -----------------------------------------------
 //   TA = 0: A stored [i][p] (lda = row length)        TA = 1: A stored [p][i]
 //   TB = 0: B stored [p][j]                           TB = 1: B stored [j][p]
 // EPI 0: C = relu(acc + bias[j])                      (forward hidden layer)
@@ -95,25 +133,27 @@ dyn_first_layer_kernel(const float* __restrict__ x_old, const float* __restrict_
 constexpr int GT_M = 64, GT_N = SS_DYN_GT_N, GT_P = 16, GT_THREADS = 256;
 constexpr int GT_CN = GT_N / 16;           // output columns per thread (4 rows x GT_CN columns)
 constexpr int GT_BL = GT_P * GT_N / GT_THREADS;   // B-tile elements staged per thread
+template <typename T>
 struct GemmEpi {
-    const float* bias;
-    const float* mask;
-    float* w;
-    float* m;
-    float* v;
-    AdamArgs adam;
+    const T* bias;
+    const T* mask;
+    T* w;
+    T* m;
+    T* v;
+    AdamArgs<T> adam;
 };
 
 // 64 x GT_N output tile, 16-deep reduction steps, 256 threads with 4 x GT_CN register micro-tiles; both
 // operand tiles are stored reduction-major in shared memory ([p][i], [p][j]) so the inner loop reads
 // one float4 of A and one of B per 16 FFMA; the next step's global loads are issued into registers
-// before the current step's FMAs (software double buffering).
-template <int TA, int TB, int EPI>
+// before the current step's FMAs (software double buffering).  T = double: the same tiling with DFMA
+// (27 KB of static shared memory).
+template <typename T, int TA, int TB, int EPI>
 __global__ void __launch_bounds__(GT_THREADS)
-dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const float* __restrict__ Bm, int ldb,
-                float* __restrict__ C, int ldc, GemmEpi e) {
-    __shared__ __align__(16) float As[2][GT_P][GT_M + 4];
-    __shared__ __align__(16) float Bs[2][GT_P][GT_N + 4];
+dyn_gemm_kernel(int M, int N, int P, const T* __restrict__ A, int lda, const T* __restrict__ Bm, int ldb,
+                T* __restrict__ C, int ldc, GemmEpi<T> e) {
+    __shared__ __align__(16) T As[2][GT_P][GT_M + 4];
+    __shared__ __align__(16) T Bs[2][GT_P][GT_N + 4];
     const int tid = threadIdx.x;
     const int i0 = blockIdx.y * GT_M, j0 = blockIdx.x * GT_N;
     const int ti = tid / 16, tj = tid % 16;          // rows ti*4.., columns tj*GT_CN..
@@ -129,17 +169,17 @@ dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const
         const int o = tid + r * GT_THREADS;
         if (TB == 0) { b_p[r] = o / GT_N; b_j[r] = o % GT_N; } else { b_j[r] = o / GT_P; b_p[r] = o % GT_P; }
     }
-    float ra[4], rb[GT_BL];
+    T ra[4], rb[GT_BL];
     auto fetch = [&](int p0) {
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             const int gi = i0 + a_i[r], gp = p0 + a_p[r];
-            ra[r] = (gi < M && gp < P) ? (TA == 0 ? __ldg(A + (size_t)gi * lda + gp) : __ldg(A + (size_t)gp * lda + gi)) : 0.f;
+            ra[r] = (gi < M && gp < P) ? (TA == 0 ? __ldg(A + (size_t)gi * lda + gp) : __ldg(A + (size_t)gp * lda + gi)) : T(0);
         }
 #pragma unroll
         for (int r = 0; r < GT_BL; ++r) {
             const int gj = j0 + b_j[r], gq = p0 + b_p[r];
-            rb[r] = (gj < N && gq < P) ? (TB == 0 ? __ldg(Bm + (size_t)gq * ldb + gj) : __ldg(Bm + (size_t)gj * ldb + gq)) : 0.f;
+            rb[r] = (gj < N && gq < P) ? (TB == 0 ? __ldg(Bm + (size_t)gq * ldb + gj) : __ldg(Bm + (size_t)gj * ldb + gq)) : T(0);
         }
     };
     auto stash = [&](int buf) {
@@ -148,7 +188,7 @@ dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const
 #pragma unroll
         for (int r = 0; r < GT_BL; ++r) Bs[buf][b_p[r]][b_j[r]] = rb[r];
     };
-    float acc[4][GT_CN] = {};
+    T acc[4][GT_CN] = {};
     fetch(0);
     stash(0);
     __syncthreads();
@@ -158,15 +198,22 @@ dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const
         if (more) fetch(p0 + GT_P);
 #pragma unroll
         for (int pp = 0; pp < GT_P; ++pp) {
-            const float4 av = *reinterpret_cast<const float4*>(&As[buf][pp][ti * 4]);
-            const float a4[4] = {av.x, av.y, av.z, av.w};
-            float b4[GT_CN];
+            T a4[4];
+            if constexpr (sizeof(T) == 4) {
+                const float4 av = *reinterpret_cast<const float4*>(&As[buf][pp][ti * 4]);
+                a4[0] = av.x; a4[1] = av.y; a4[2] = av.z; a4[3] = av.w;
+            } else {
+                const double2 a01 = *reinterpret_cast<const double2*>(&As[buf][pp][ti * 4]);
+                const double2 a23 = *reinterpret_cast<const double2*>(&As[buf][pp][ti * 4 + 2]);
+                a4[0] = a01.x; a4[1] = a01.y; a4[2] = a23.x; a4[3] = a23.y;
+            }
+            T b4[GT_CN];
 #pragma unroll
             for (int cidx = 0; cidx < GT_CN; ++cidx) b4[cidx] = Bs[buf][pp][tj * GT_CN + cidx];
 #pragma unroll
             for (int r = 0; r < 4; ++r)
 #pragma unroll
-                for (int cidx = 0; cidx < GT_CN; ++cidx) acc[r][cidx] = fmaf(a4[r], b4[cidx], acc[r][cidx]);
+                for (int cidx = 0; cidx < GT_CN; ++cidx) acc[r][cidx] = fma_t(a4[r], b4[cidx], acc[r][cidx]);
         }
         if (more) {
             stash(buf ^ 1);
@@ -182,14 +229,14 @@ dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const
         for (int cidx = 0; cidx < GT_CN; ++cidx) {
             const int gj = j0 + tj * GT_CN + cidx;
             if (gj >= N) continue;
-            const float a = acc[r][cidx];
+            const T a = acc[r][cidx];
             if (EPI == 0) {
-                C[(size_t)gi * ldc + gj] = fmaxf(a + e.bias[gj], 0.f);
+                C[(size_t)gi * ldc + gj] = relu_t(a + e.bias[gj]);
             } else if (EPI == 1) {
-                C[(size_t)gi * ldc + gj] = e.mask[(size_t)gi * ldc + gj] > 0.f ? a : 0.f;
+                C[(size_t)gi * ldc + gj] = e.mask[(size_t)gi * ldc + gj] > T(0) ? a : T(0);
             } else {
                 const size_t o = (size_t)gi * ldc + gj;
-                float w = e.w[o], m = e.m[o], v = e.v[o];
+                T w = e.w[o], m = e.m[o], v = e.v[o];
                 adam_update(a, w, m, v, e.adam);
                 e.w[o] = w; e.m[o] = m; e.v[o] = v;
             }
@@ -201,27 +248,28 @@ dyn_gemm_kernel(int M, int N, int P, const float* __restrict__ A, int lda, const
 // out[b][j] = H[b] . W[:, j] + bias[j]; dOut = 2 (out - z) / (B dout); loss = mean (out - z)^2;
 // when training also dH[b][k] = (sum_j dOut[b][j] W[k][j]) * [H[b][k] > 0] (N = dout is tiny).
 // one warp per batch row; per-block partial loss -> last block (ticket) sums them in fixed order
+template <typename T>
 __global__ void __launch_bounds__(256)
-dyn_out_loss_kernel(const float* __restrict__ H, int h, const float* __restrict__ W, const float* __restrict__ bias,
-                    const float* __restrict__ Z, int B, int dout, float* __restrict__ dOut, float* __restrict__ dH,
+dyn_out_loss_kernel(const T* __restrict__ H, int h, const T* __restrict__ W, const T* __restrict__ bias,
+                    const T* __restrict__ Z, int B, int dout, T* __restrict__ dOut, T* __restrict__ dH,
                     double* __restrict__ partial, unsigned int* __restrict__ ticket, double* __restrict__ loss_out,
                     int train) {
     __shared__ double s_part[8];
-    __shared__ float s_dout[8][SS_MAX_D];
+    __shared__ T s_dout[8][SS_MAX_D];
     __shared__ bool s_last;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * 8 + warp;
     double sq = 0.0;
     if (b < B) {
-        const float* hb = H + (size_t)b * h;
+        const T* hb = H + (size_t)b * h;
         for (int j = 0; j < dout; ++j) {
-            float acc = 0.f;
-            for (int k = lane; k < h; k += 32) acc = fmaf(hb[k], W[(size_t)k * dout + j], acc);
+            T acc = T(0);
+            for (int k = lane; k < h; k += 32) acc = fma_t(hb[k], W[(size_t)k * dout + j], acc);
             for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-            const float out = acc + bias[j];
-            const float diff = out - Z[(size_t)b * dout + j];
+            const T out = acc + bias[j];
+            const T diff = out - Z[(size_t)b * dout + j];
             if (lane == 0) {
-                const float g = 2.f * diff / (float)(B * dout);
+                const T g = T(2) * diff / (T)(B * dout);
                 if (train) dOut[(size_t)b * dout + j] = g;
                 s_dout[warp][j] = g;
                 sq += (double)diff * (double)diff;
@@ -230,9 +278,9 @@ dyn_out_loss_kernel(const float* __restrict__ H, int h, const float* __restrict_
         if (train) {
             __syncwarp();
             for (int k = lane; k < h; k += 32) {
-                float acc = 0.f;
-                for (int j = 0; j < dout; ++j) acc = fmaf(s_dout[warp][j], W[(size_t)k * dout + j], acc);
-                dH[(size_t)b * h + k] = hb[k] > 0.f ? acc : 0.f;
+                T acc = T(0);
+                for (int j = 0; j < dout; ++j) acc = fma_t(s_dout[warp][j], W[(size_t)k * dout + j], acc);
+                dH[(size_t)b * h + k] = hb[k] > T(0) ? acc : T(0);
             }
         }
     }
@@ -259,37 +307,40 @@ dyn_out_loss_kernel(const float* __restrict__ H, int h, const float* __restrict_
 // (dW[k][j] = sum_b A[b][k] dY[b][j] with a tiny K or N) and all bias vectors (column sums of dY),
 // each followed by its Adam update.  One warp per parameter: lanes stride over the batch, shuffle
 // tree (fixed order).
+template <typename T>
 struct SmallSeg {
-    const float* A;      // [B][lda] activations, or null for a bias (A = 1)
-    const float* dY;     // [B][ldy]
-    float* w;
-    float* m;
-    float* v;
+    const T* A;          // [B][lda] activations, or null for a bias (A = 1)
+    const T* dY;         // [B][ldy]
+    T* w;
+    T* m;
+    T* v;
     int lda, ldy, N;     // parameter o of the segment: k = o / N, j = o % N
     int start;           // first warp of the segment
 };
+template <typename T>
 struct SmallJob {
-    SmallSeg seg[DYN_MAX_LAYERS + 3];
+    SmallSeg<T> seg[DYN_MAX_LAYERS + 3];
     int n_seg, total;
 };
+template <typename T>
 __global__ void __launch_bounds__(256)
-dyn_small_updates_kernel(SmallJob job, int B, AdamArgs adam) {
+dyn_small_updates_kernel(SmallJob<T> job, int B, AdamArgs<T> adam) {
     const int wid = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (wid >= job.total) return;
     int si = 0;
     while (si + 1 < job.n_seg && wid >= job.seg[si + 1].start) ++si;
-    const SmallSeg& g = job.seg[si];
+    const SmallSeg<T>& g = job.seg[si];
     const int o = wid - g.start, k = o / g.N, j = o % g.N;
-    float acc = 0.f;
+    T acc = T(0);
     if (g.A) {
-        for (int b = lane; b < B; b += 32) acc = fmaf(g.A[(size_t)b * g.lda + k], g.dY[(size_t)b * g.ldy + j], acc);
+        for (int b = lane; b < B; b += 32) acc = fma_t(g.A[(size_t)b * g.lda + k], g.dY[(size_t)b * g.ldy + j], acc);
     } else {
         for (int b = lane; b < B; b += 32) acc += g.dY[(size_t)b * g.ldy + j];
     }
     for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
     if (lane == 0) {
-        float w = g.w[o], m = g.m[o], v = g.v[o];
+        T w = g.w[o], m = g.m[o], v = g.v[o];
         adam_update(acc, w, m, v, adam);
         g.w[o] = w; g.m[o] = m; g.v[o] = v;
     }
@@ -301,6 +352,12 @@ __global__ void dyn_pack_fp32_kernel(const float* __restrict__ W, const float* _
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
     if (o < in * out) Wp[(size_t)(o / out) * out_pad + (o % out)] = W[o];
     if (o < out) bp[o] = b[o];
+}
+
+// float64 masters rounded once to float: the source of the FP32 and tcgen05 images after FP64 training
+__global__ void dyn_round_kernel(const double* __restrict__ src, float* __restrict__ dst, size_t n) {
+    const size_t o = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+    if (o < n) dst[o] = (float)src[o];
 }
 
 __device__ __forceinline__ unsigned short bf16_bits_dev(float f) {
@@ -394,22 +451,25 @@ static DynLayout dyn_layout(const ss_ctx* c) {
     return y;
 }
 
-// (re)create the FP32 master copy + zeroed Adam state from the float64 host parameters of
-// ss_mpc_set_model; called lazily by the first training call after a host-side set_model
+// (re)create the master copy (T = float: FP32 trainer, double: SS_PRECISION_FP64) + zeroed Adam state
+// from the float64 host parameters of ss_mpc_set_model; called lazily by the first training call after
+// a host-side set_model
+template <typename T>
 static int dyn_sync_from_host(ss_ctx* c) {
     const DynLayout y = dyn_layout(c);
-    std::vector<float> host(y.total, 0.f);
+    const size_t bytes = y.total * sizeof(T);
+    std::vector<T> host(y.total, T(0));
     for (int l = 0; l <= y.L; ++l) {
-        for (size_t i = 0; i < (size_t)y.in[l] * y.out[l]; ++i) host[y.w_off[l] + i] = (float)c->hw[l][i];
-        for (int i = 0; i < y.out[l]; ++i) host[y.b_off[l] + i] = (float)c->hb[l][i];
+        for (size_t i = 0; i < (size_t)y.in[l] * y.out[l]; ++i) host[y.w_off[l] + i] = (T)c->hw[l][i];
+        for (int i = 0; i < y.out[l]; ++i) host[y.b_off[l] + i] = (T)c->hb[l][i];
     }
-    SS_CUDA_CHECK(c, c->dyn_params.ensure(y.total * 4));
-    SS_CUDA_CHECK(c, c->dyn_m.ensure(y.total * 4));
-    SS_CUDA_CHECK(c, c->dyn_v.ensure(y.total * 4));
-    SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_params.p, host.data(), y.total * 4, cudaMemcpyHostToDevice, c->stream));
+    SS_CUDA_CHECK(c, c->dyn_params.ensure(bytes));
+    SS_CUDA_CHECK(c, c->dyn_m.ensure(bytes));
+    SS_CUDA_CHECK(c, c->dyn_v.ensure(bytes));
+    SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_params.p, host.data(), bytes, cudaMemcpyHostToDevice, c->stream));
     if (!c->dyn_adam_valid) {
-        SS_CUDA_CHECK(c, cudaMemsetAsync(c->dyn_m.p, 0, y.total * 4, c->stream));
-        SS_CUDA_CHECK(c, cudaMemsetAsync(c->dyn_v.p, 0, y.total * 4, c->stream));
+        SS_CUDA_CHECK(c, cudaMemsetAsync(c->dyn_m.p, 0, bytes, c->stream));
+        SS_CUDA_CHECK(c, cudaMemsetAsync(c->dyn_v.p, 0, bytes, c->stream));
         c->dyn_t = 0;
         c->dyn_adam_valid = true;
     }
@@ -418,24 +478,29 @@ static int dyn_sync_from_host(ss_ctx* c) {
     return SS_OK;
 }
 
+template <typename T>
+static int dyn_upload_data(ss_ctx* c, int which, const double* X, const double* Z, int64_t n_rows) {
+    const int din = c->d + c->da, dout = c->d;
+    std::vector<T> x((size_t)n_rows * din), z((size_t)n_rows * dout);
+    for (size_t i = 0; i < x.size(); ++i) x[i] = (T)X[i];
+    for (size_t i = 0; i < z.size(); ++i) z[i] = (T)Z[i];
+    SS_CUDA_CHECK(c, c->dyn_x[which].ensure(x.size() * sizeof(T) + 16));
+    SS_CUDA_CHECK(c, c->dyn_z[which].ensure(z.size() * sizeof(T) + 16));
+    if (n_rows > 0) {
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_x[which].p, x.data(), x.size() * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_z[which].p, z.data(), z.size() * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+    }
+    c->dyn_rows[which] = n_rows;
+    return SS_OK;
+}
+
 extern "C" int ss_dyn_set_data(ss_ctx* c, int which, const double* X, const double* Z, int64_t n_rows) {
     if (!c) return SS_EINVAL;
     if (!c->model_set) SS_FAIL(c, SS_ESTATE, "dyn: set the model first (ss_mpc_set_model)");
     if ((which != 0 && which != 1) || n_rows < 0 || (n_rows > 0 && (!X || !Z))) SS_FAIL(c, SS_EINVAL, "dyn: bad data arguments");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
-    const int din = c->d + c->da, dout = c->d;
-    std::vector<float> x((size_t)n_rows * din), z((size_t)n_rows * dout);
-    for (size_t i = 0; i < x.size(); ++i) x[i] = (float)X[i];
-    for (size_t i = 0; i < z.size(); ++i) z[i] = (float)Z[i];
-    SS_CUDA_CHECK(c, c->dyn_x[which].ensure(x.size() * 4 + 16));
-    SS_CUDA_CHECK(c, c->dyn_z[which].ensure(z.size() * 4 + 16));
-    if (n_rows > 0) {
-        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_x[which].p, x.data(), x.size() * 4, cudaMemcpyHostToDevice, c->stream));
-        SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_z[which].p, z.data(), z.size() * 4, cudaMemcpyHostToDevice, c->stream));
-        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
-    }
-    c->dyn_rows[which] = n_rows;
-    return SS_OK;
+    return c->dyn_fp64 ? dyn_upload_data<double>(c, which, X, Z, n_rows) : dyn_upload_data<float>(c, which, X, Z, n_rows);
 }
 
 extern "C" int ss_dyn_reset_optimizer(ss_ctx* c) {
@@ -445,54 +510,70 @@ extern "C" int ss_dyn_reset_optimizer(ss_ctx* c) {
     return SS_OK;
 }
 
-template <int TA, int TB, int EPI>
-static void launch_gemm(ss_ctx* c, int M, int N, int P, const float* A, int lda, const float* B, int ldb, float* C,
-                        int ldc, const GemmEpi& e) {
+extern "C" int ss_dyn_set_precision(ss_ctx* c, int precision) {
+    if (!c) return SS_EINVAL;
+    if (precision != SS_PRECISION_FP32 && precision != SS_PRECISION_FP64)
+        SS_FAIL(c, SS_EINVAL, "dyn: the trainer's precision is SS_PRECISION_FP32 or SS_PRECISION_FP64");
+    const bool fp64 = precision == SS_PRECISION_FP64;
+    if (fp64 == c->dyn_fp64) return SS_OK;
+    // the buffers change their element type: nothing in them survives
+    c->dyn_fp64 = fp64;
+    c->dyn_adam_valid = false;
+    c->dyn_params_valid = false;
+    c->dyn_dirty = false;
+    c->dyn_rows[0] = c->dyn_rows[1] = 0;
+    return SS_OK;
+}
+
+template <typename T, int TA, int TB, int EPI>
+static void launch_gemm(ss_ctx* c, int M, int N, int P, const T* A, int lda, const T* B, int ldb, T* C, int ldc,
+                        const GemmEpi<T>& e) {
     dim3 grid((N + GT_N - 1) / GT_N, (M + GT_M - 1) / GT_M);
-    dyn_gemm_kernel<TA, TB, EPI><<<grid, GT_THREADS, 0, c->stream>>>(M, N, P, A, lda, B, ldb, C, ldc, e);
+    dyn_gemm_kernel<T, TA, TB, EPI><<<grid, GT_THREADS, 0, c->stream>>>(M, N, P, A, lda, B, ldb, C, ldc, e);
     c->launches++;
 }
 
 // one batch through the network: forward (+ loss) and, when train != 0, backward + Adam
+template <typename T>
 static int dyn_step(ss_ctx* c, const DynLayout& y, const int* idx_old, const int* idx_new, int n_old, int B,
-                    double* loss_out, int train, float lr, int src_old, int src_new) {
-    float* P = c->dyn_params.as<float>();
-    float* Mo = c->dyn_m.as<float>();
-    float* Vo = c->dyn_v.as<float>();
+                    double* loss_out, int train, T lr, int src_old, int src_new) {
+    T* P = c->dyn_params.as<T>();
+    T* Mo = c->dyn_m.as<T>();
+    T* Vo = c->dyn_v.as<T>();
     const int h = y.h, din = y.din, dout = y.dout, L = y.L;
     // activations: X [B][din], Z [B][dout], H_1..H_L [B][h]; gradients dOut [B][dout], dH_1..dH_L [B][h]
-    float* X = c->dyn_act.as<float>();
-    float* Z = X + (size_t)B * din;
-    float* H = Z + (size_t)B * dout;                          // H_l at H + (l - 1) * B * h
-    float* dOut = H + (size_t)L * B * h;
-    float* dH = dOut + (size_t)B * dout;                      // dH_l at dH + (l - 1) * B * h
+    T* X = c->dyn_act.as<T>();
+    T* Z = X + (size_t)B * din;
+    T* H = Z + (size_t)B * dout;                              // H_l at H + (l - 1) * B * h
+    T* dOut = H + (size_t)L * B * h;
+    T* dH = dOut + (size_t)B * dout;                          // dH_l at dH + (l - 1) * B * h
     double* partial = c->dyn_scratch.as<double>();
     unsigned int* ticket = reinterpret_cast<unsigned int*>(partial + 256);
-    AdamArgs adam;
-    adam.beta1 = 0.9f; adam.beta2 = 0.999f; adam.eps = 1e-8f;
-    adam.omb1 = (float)(1.0 - 0.9); adam.omb2 = (float)(1.0 - 0.999);
+    AdamArgs<T> adam;
+    adam.beta1 = (T)0.9; adam.beta2 = (T)0.999; adam.eps = (T)1e-8;
+    adam.omb1 = (T)(1.0 - 0.9); adam.omb2 = (T)(1.0 - 0.999);
     if (train) {
         c->dyn_t += 1;
         const double t = (double)c->dyn_t;
-        adam.lr_t = (float)((double)lr * std::sqrt(1.0 - std::pow(0.999, t)) / (1.0 - std::pow(0.9, t)));
+        adam.lr_t = (T)((double)lr * std::sqrt(1.0 - std::pow(0.999, t)) / (1.0 - std::pow(0.9, t)));
     } else {
-        adam.lr_t = 0.f;
+        adam.lr_t = T(0);
     }
     const int rows_pb = 8;
-    dyn_first_layer_kernel<<<(B + rows_pb - 1) / rows_pb, rows_pb * 32, (size_t)rows_pb * din * 4, c->stream>>>(
-        c->dyn_x[src_old].as<float>(), c->dyn_z[src_old].as<float>(), c->dyn_x[src_new].as<float>(),
-        c->dyn_z[src_new].as<float>(), idx_old, idx_new, n_old, B, din, dout, P + y.w_off[0], P + y.b_off[0], h, 1, X, Z, H);
+    dyn_first_layer_kernel<T><<<(B + rows_pb - 1) / rows_pb, rows_pb * 32, (size_t)rows_pb * din * sizeof(T), c->stream>>>(
+        c->dyn_x[src_old].as<T>(), c->dyn_z[src_old].as<T>(), c->dyn_x[src_new].as<T>(),
+        c->dyn_z[src_new].as<T>(), idx_old, idx_new, n_old, B, din, dout, P + y.w_off[0], P + y.b_off[0], h, 1, X, Z, H);
     c->launches++;
-    GemmEpi e;
+    GemmEpi<T> e;
     std::memset(&e, 0, sizeof(e));
     for (int l = 1; l < L; ++l) {
         e.bias = P + y.b_off[l];
-        launch_gemm<0, 0, 0>(c, B, h, h, H + (size_t)(l - 1) * B * h, h, P + y.w_off[l], h, H + (size_t)l * B * h, h, e);
+        launch_gemm<T, 0, 0, 0>(c, B, h, h, H + (size_t)(l - 1) * B * h, h, P + y.w_off[l], h, H + (size_t)l * B * h, h, e);
     }
-    const float* HL = H + (size_t)(L - 1) * B * h;
-    float* dHL = dH + (size_t)(L - 1) * B * h;
-    dyn_out_loss_kernel<<<(B + 7) / 8, 256, 0, c->stream>>>(HL, h, P + y.w_off[L], P + y.b_off[L], Z, B, dout, dOut, dHL,
-                                                            partial, ticket, loss_out, train);
+    const T* HL = H + (size_t)(L - 1) * B * h;
+    T* dHL = dH + (size_t)(L - 1) * B * h;
+    dyn_out_loss_kernel<T><<<(B + 7) / 8, 256, 0, c->stream>>>(HL, h, P + y.w_off[L], P + y.b_off[L], Z, B, dout, dOut,
+                                                               dHL, partial, ticket, loss_out, train);
     c->launches++;
     if (!train) {
         SS_CUDA_CHECK(c, cudaGetLastError());
@@ -503,17 +584,17 @@ static int dyn_step(ss_ctx* c, const DynLayout& y, const int* idx_old, const int
     for (int l = L - 1; l >= 1; --l) {
         // dH_l [B][h] = dH_{l+1} [B][h] W_l^T (W_l stored [in = h][out = h]) (.) [H_l > 0]
         e.mask = H + (size_t)(l - 1) * B * h;
-        launch_gemm<0, 1, 1>(c, B, h, h, dH + (size_t)l * B * h, h, P + y.w_off[l], h, dH + (size_t)(l - 1) * B * h, h, e);
+        launch_gemm<T, 0, 1, 1>(c, B, h, h, dH + (size_t)l * B * h, h, P + y.w_off[l], h, dH + (size_t)(l - 1) * B * h, h, e);
         // dW_l [h][h] = H_l^T [h][B] dH_{l+1} [B][h], Adam fused
         e.w = P + y.w_off[l]; e.m = Mo + y.w_off[l]; e.v = Vo + y.w_off[l]; e.adam = adam;
-        launch_gemm<1, 0, 2>(c, h, h, B, H + (size_t)(l - 1) * B * h, h, dH + (size_t)l * B * h, h, nullptr, h, e);
+        launch_gemm<T, 1, 0, 2>(c, h, h, B, H + (size_t)(l - 1) * B * h, h, dH + (size_t)l * B * h, h, nullptr, h, e);
     }
     // first / last layer matrices and every bias vector: one launch
-    SmallJob job;
+    SmallJob<T> job;
     std::memset(&job, 0, sizeof(job));
     int ns = 0, start = 0;
-    auto add_seg = [&](const float* A, int lda, const float* dY, int ldy, int K, int N, size_t off) {
-        SmallSeg& g = job.seg[ns++];
+    auto add_seg = [&](const T* A, int lda, const T* dY, int ldy, int K, int N, size_t off) {
+        SmallSeg<T>& g = job.seg[ns++];
         g.A = A; g.lda = lda; g.dY = dY; g.ldy = ldy; g.N = N;
         g.w = P + off; g.m = Mo + off; g.v = Vo + off;
         g.start = start;
@@ -525,7 +606,7 @@ static int dyn_step(ss_ctx* c, const DynLayout& y, const int* idx_old, const int
         add_seg(nullptr, 0, l == L ? dOut : dH + (size_t)l * B * h, y.out[l], 1, y.out[l], y.b_off[l]);
     job.n_seg = ns;
     job.total = start;
-    dyn_small_updates_kernel<<<(start + 7) / 8, 256, 0, c->stream>>>(job, B, adam);
+    dyn_small_updates_kernel<T><<<(start + 7) / 8, 256, 0, c->stream>>>(job, B, adam);
     c->launches++;
     SS_CUDA_CHECK(c, cudaGetLastError());
     return SS_OK;
@@ -536,11 +617,11 @@ static int dyn_prepare(ss_ctx* c, int B) {
     if (B < 1) SS_FAIL(c, SS_EINVAL, "dyn: empty batch");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     if (!c->dyn_params_valid) {
-        int rc = dyn_sync_from_host(c);
+        int rc = c->dyn_fp64 ? dyn_sync_from_host<double>(c) : dyn_sync_from_host<float>(c);
         if (rc) return rc;
     }
     const DynLayout y = dyn_layout(c);
-    const size_t act = ((size_t)B * (y.din + 2 * y.dout) + 2 * (size_t)y.L * B * y.h) * 4;
+    const size_t act = ((size_t)B * (y.din + 2 * y.dout) + 2 * (size_t)y.L * B * y.h) * (c->dyn_fp64 ? 8 : 4);
     SS_CUDA_CHECK(c, c->dyn_act.ensure(act));
     if (!c->dyn_scratch.p) {
         SS_CUDA_CHECK(c, c->dyn_scratch.ensure(256 * 8 + 64));
@@ -573,8 +654,11 @@ extern "C" int ss_dyn_train_batches(ss_ctx* c, const int32_t* idx_old, const int
     if (n_new) SS_CUDA_CHECK(c, cudaMemcpyAsync(d_new, idx_new, (size_t)n_batches * n_new * 4, cudaMemcpyHostToDevice, c->stream));
     timer_begin(c);
     for (int i = 0; i < n_batches; ++i) {
-        rc = dyn_step(c, y, d_old + (size_t)i * n_old, d_new + (size_t)i * n_new, n_old, B, c->dyn_losses.as<double>() + i, 1,
-                      (float)lr, 0, 1);
+        int* io = d_old + (size_t)i * n_old;
+        int* inw = d_new + (size_t)i * n_new;
+        double* li = c->dyn_losses.as<double>() + i;
+        rc = c->dyn_fp64 ? dyn_step<double>(c, y, io, inw, n_old, B, li, 1, lr, 0, 1)
+                         : dyn_step<float>(c, y, io, inw, n_old, B, li, 1, (float)lr, 0, 1);
         if (rc) return rc;
     }
     timer_mark(c, "dyn_train");
@@ -604,8 +688,10 @@ extern "C" int ss_dyn_eval_loss(ss_ctx* c, int which, int batchsize, double* out
     SS_CUDA_CHECK(c, c->dyn_losses.ensure((size_t)nb * 8));
     SS_CUDA_CHECK(c, cudaMemcpyAsync(c->dyn_idx.p, idx.data(), idx.size() * 4, cudaMemcpyHostToDevice, c->stream));
     for (int i = 0; i < nb; ++i) {
-        rc = dyn_step(c, y, c->dyn_idx.as<int>() + (size_t)i * batchsize, nullptr, batchsize, batchsize,
-                      c->dyn_losses.as<double>() + i, 0, 0.f, which, which);
+        int* io = c->dyn_idx.as<int>() + (size_t)i * batchsize;
+        double* li = c->dyn_losses.as<double>() + i;
+        rc = c->dyn_fp64 ? dyn_step<double>(c, y, io, nullptr, batchsize, batchsize, li, 0, 0.0, which, which)
+                         : dyn_step<float>(c, y, io, nullptr, batchsize, batchsize, li, 0, 0.f, which, which);
         if (rc) return rc;
     }
     std::vector<double> l(nb);
@@ -631,6 +717,16 @@ extern "C" int ss_dyn_get_params(ss_ctx* c, double* const* out_weights, double* 
         }
         return SS_OK;
     }
+    if (c->dyn_fp64) {                // the float64 masters as they are
+        std::vector<double> host(y.total);
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(host.data(), c->dyn_params.p, y.total * 8, cudaMemcpyDeviceToHost, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+        for (int l = 0; l <= y.L; ++l) {
+            std::memcpy(out_weights[l], host.data() + y.w_off[l], (size_t)y.in[l] * y.out[l] * 8);
+            std::memcpy(out_biases[l], host.data() + y.b_off[l], (size_t)y.out[l] * 8);
+        }
+        return SS_OK;
+    }
     std::vector<float> host(y.total);
     SS_CUDA_CHECK(c, cudaMemcpyAsync(host.data(), c->dyn_params.p, y.total * 4, cudaMemcpyDeviceToHost, c->stream));
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
@@ -648,7 +744,15 @@ extern "C" int ss_dyn_commit(ss_ctx* c) {
     if (!c->dyn_params_valid || !c->dyn_dirty) return SS_OK;
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     const DynLayout y = dyn_layout(c);
+    // the FP32 and tcgen05 images come from FP32 parameters: after FP64 training, the masters rounded once
     const float* P = c->dyn_params.as<float>();
+    if (c->dyn_fp64) {
+        SS_CUDA_CHECK(c, c->dyn_round.ensure(y.total * 4));
+        dyn_round_kernel<<<(unsigned)((y.total + 255) / 256), 256, 0, c->stream>>>(c->dyn_params.as<double>(),
+                                                                                  c->dyn_round.as<float>(), y.total);
+        c->launches++;
+        P = c->dyn_round.as<float>();
+    }
     for (int l = 0; l <= y.L; ++l) {
         const int out_pad = l == y.L ? (c->d + 7) / 8 * 8 : c->h_pad;
         const int n = std::max(y.in[l] * y.out[l], y.out[l]);
@@ -656,9 +760,18 @@ extern "C" int ss_dyn_commit(ss_ctx* c) {
                                                                     out_pad, c->w32[l].as<float>(), c->b32[l].as<float>());
         c->launches++;
     }
-    // the float64 copies of SS_PRECISION_FP64 roll out the same (widened) parameters Dyn_Model.export() returns
+    // the float64 copies of SS_PRECISION_FP64 roll out the same parameters Dyn_Model.export() returns: the
+    // float64 masters unchanged, or the FP32 masters widened
     for (int l = 0; l <= y.L; ++l) {
         const int out_pad = l == y.L ? (c->d + 7) / 8 * 8 : c->h_pad;
+        if (c->dyn_fp64) {
+            const double* P64 = c->dyn_params.as<double>();
+            SS_CUDA_CHECK(c, cudaMemcpy2DAsync(c->w64[l].p, (size_t)out_pad * 8, P64 + y.w_off[l], (size_t)y.out[l] * 8,
+                                               (size_t)y.out[l] * 8, y.in[l], cudaMemcpyDeviceToDevice, c->stream));
+            SS_CUDA_CHECK(c, cudaMemcpyAsync(c->b64[l].p, P64 + y.b_off[l], (size_t)y.out[l] * 8, cudaMemcpyDeviceToDevice,
+                                             c->stream));
+            continue;
+        }
         int rc = mpc_fp64_widen(c, P + y.w_off[l], P + y.b_off[l], y.in[l], y.out[l], out_pad, c->w64[l].as<double>(),
                                 c->b64[l].as<double>());
         if (rc) return rc;

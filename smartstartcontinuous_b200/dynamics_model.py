@@ -8,7 +8,9 @@ the CUDA engine: ``train`` uploads the two data sets once, draws the batch row i
 reference's numpy calls (same stream of ``npr`` draws, hence the same batches for the same seed)
 and runs every epoch's Adam steps on the device (csrc/dyn_train.cu, one index upload and one loss
 read-back per epoch, no host copy of a batch); the trained parameters are handed to the rollout
-kernels on the device (``Engine.dyn_commit``).  ``do_forward_sim`` keeps the reference's signature
+kernels on the device (``Engine.dyn_commit``).  ``precision="fp64"`` trains in float64 like the
+reference's graph (data, parameters, Adam moments and every step), so the weights stay the reference's
+up to the summation order of the GEMMs; the default "fp32" is the faster FP32 trainer.  ``do_forward_sim`` keeps the reference's signature
 and runs on the engine as well.  There is no CPU path: a missing engine raises.
 """
 from __future__ import annotations
@@ -35,9 +37,13 @@ def _xavier_normal(rng, shape, fan_in, fan_out):
 class Dyn_Model:
     def __init__(self, inputSize, outputSize, sess, learning_rate, batchsize, num_fc_layers,
                  depth_fc_layers, mean_x, mean_y, mean_z, std_x, std_y, std_z, tf_datatype, verbose,
-                 engine=None, seed=None):
+                 engine=None, seed=None, *, precision="fp32"):
+        """precision: arithmetic of the device trainer, "fp32" or "fp64" (the reference's float64; set on the
+        engine here, before the initial weights).  tf_datatype is accepted and unused."""
         if engine is None:
             raise RuntimeError("Dyn_Model needs a CUDA engine (there is no CPU implementation of this path)")
+        engine.dyn_set_precision(precision)
+        self.precision = precision
         self.sess = sess                      # accepted for signature compatibility, unused
         self.batchsize = batchsize
         self.inputSize = inputSize

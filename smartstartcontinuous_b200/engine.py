@@ -416,6 +416,16 @@ class Engine:
     def dyn_reset_optimizer(self):
         self._check(self._lib.ss_dyn_reset_optimizer(self._h))
 
+    def dyn_set_precision(self, precision):
+        """Arithmetic of the device trainer: "fp32" (default) or "fp64" (float64 data, masters, moments
+        and steps, like the reference's graph).  A change discards the trainer state: training restarts
+        from the parameters of the last set_model with fresh Adam moments, and both data sets must be
+        uploaded again."""
+        codes = {"fp32": PRECISION_FP32, "fp64": PRECISION_FP64}
+        if precision not in codes:
+            raise ValueError("trainer precision must be 'fp32' or 'fp64', got %r" % (precision,))
+        self._check(self._lib.ss_dyn_set_precision(self._h, codes[precision]))
+
     def dyn_get_params(self):
         """(weights, biases) of the model as float64 numpy ([in, out] / [out])."""
         d, da, L, h = self._model_shape

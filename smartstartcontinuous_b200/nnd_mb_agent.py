@@ -18,6 +18,10 @@ Extra keyword-only options (all default to the reference behaviour):
                       reference (its decision up to the summation order of the GEMMs and reductions, also
                       when the best two scores are closer than the FP32 / BF16 tolerances), several times
                       slower than "bf16_tc"; "auto" never picks it
+  train_precision     "fp32" | "fp64"; arithmetic of the device trainer behind train_dynamics_model.  "fp64"
+                      trains in float64 like the reference's graph, so a retrained model stays the reference's
+                      up to the summation order of the GEMMs; the reference-faithful configuration is
+                      precision="fp64", train_precision="fp64"
   device_sampling     False: the actions of numpy.random.uniform exactly like :500-501 -- the global
                       MT19937 stream, generated on the GPU from np.random.get_state() and advanced with
                       set_state (host_rng=True draws them on the host and uploads them instead, False
@@ -118,7 +122,7 @@ class NND_MB_agent(NavigationRLAgent):
 
                  *, engine=None, device=0, penalty_mode="reference", precision="auto",
                  device_sampling=False, host_rng=None, training_data=None, model_root=None, seed=None,
-                 planner=None):
+                 planner=None, train_precision="fp32"):
         self.theta = 1            # distance function is scaled instead (NND_MB_agent.py:135-138)
         self.final_steps = final_steps
         self.gamma = gamma
@@ -221,7 +225,7 @@ class NND_MB_agent(NavigationRLAgent):
         self.dyn_model = Dyn_Model(self.inputs.shape[1], self.outputs.shape[1], self.sess, lr, batchsize,
                                    num_fc_layers, depth_fc_layers, self.mean_x, self.mean_y, self.mean_z,
                                    self.std_x, self.std_y, self.std_z, self.tf_datatype, verbose,
-                                   engine=self.engine, seed=seed)
+                                   engine=self.engine, seed=seed, precision=train_precision)
         self.dyn_model.push_to_engine()
         # the default decision path draws numpy's stream on the GPU: build its jump-ahead plan now, not in the
         # first decision
