@@ -113,6 +113,15 @@ int ss_kde_ucb_argmax_dev(ss_ctx* ctx, const double* data_dev, int64_t n_pts, in
                           int64_t n_transitions, double volume, double alpha, double beta,
                           double* out_density_dev, double* out_ucb_dev,
                           int64_t* out_best_j, double* out_best_ucb);
+/* precision of the selection (all three ss_kde_ucb_argmax* entry points; signatures, errors and outputs
+ * unchanged): SS_PRECISION_FP32 (default; FP32 / tcgen05 pair stage, densities to ~1e-5) or SS_PRECISION_FP64,
+ * which follows scipy.stats.gaussian_kde 1.18 operation for operation in float64 (two-pass weighted
+ * covariance, Cholesky times the Scott factor, triangular solves, sum_i w * (exp(-|P_i - Z_j|^2 / 2) * norm))
+ * and forms alpha * values in float32 as numpy does with the float32 values: densities agree with scipy to
+ * ~1e-13 relative, so the choice is scipy's whenever the top-two UCB gap is larger than that.  The mirror entry
+ * point then fits from the mirror's rows, not from its running moments.  A query's density does not depend on
+ * the batch it is evaluated in.  Setting the current value is a no-op; any other value: SS_EINVAL. */
+int ss_kde_set_precision(ss_ctx* ctx, int precision);
 
 /* ---- stage 2: NND_MB random-shooting MPC ---------------------------------------------
  * ss_mpc_set_model: the weights Dyn_Model holds (dynamics_model.py:36-37,

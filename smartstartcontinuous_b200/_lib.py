@@ -50,6 +50,7 @@ SIGNATURES = {
     "ss_kde_ucb_argmax_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
                                         C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,
                                         C.c_void_p, C.c_void_p, _c_int64_p, _c_double_p]),
+    "ss_kde_set_precision": (C.c_int, [C.c_void_p, C.c_int]),
     "ss_mpc_set_model": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)] + [C.c_void_p] * 6),
     "ss_mpc_set_plan": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libss_b200.so")
-SOURCES = ["capi.cu", "kde.cu", "mpc_host.cu", "mpc_simt.cu", "mpc_score.cu", "mpc_tc.cu", "mpc_tc_quad.cu", "mpc_fp64.cu", "plan_geom.cu", "value_net.cu", "peer.cu", "dyn_train.cu", "mt19937.cu", "py_random.cu"]
+SOURCES = ["capi.cu", "kde.cu", "kde_fp64.cu", "mpc_host.cu", "mpc_simt.cu", "mpc_score.cu", "mpc_tc.cu", "mpc_tc_quad.cu", "mpc_fp64.cu", "plan_geom.cu", "value_net.cu", "peer.cu", "dyn_train.cu", "mt19937.cu", "py_random.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"] + os.environ.get("SS_NVCC_EXTRA", "").split()
 

@@ -437,9 +437,9 @@ extern "C" int ss_kde_ucb_argmax_mirror(ss_ctx* c, int64_t count, int64_t last_r
         ucb_dev = c->kde_ucb.as<double>();
     }
     // the estimator is fitted from the running moments of the buffer rows; they are recomputed exactly after a
-    // bulk upload and once per buffer turnover
+    // bulk upload and once per buffer turnover (SS_PRECISION_FP64 fits from the rows themselves, in two passes)
     const double* sums = nullptr;
-    if (c->mirror_filled == count && !getenv("SS_MIRROR_NO_RUNNING_MOMENTS")) {
+    if (c->mirror_filled == count && !c->kde_fp64 && !getenv("SS_MIRROR_NO_RUNNING_MOMENTS")) {
         const int nm = d + d * (d + 1) / 2;
         if (!c->mirror_mom_valid) {
             SS_CUDA_CHECK(c, c->mirror_mom.ensure((size_t)(nm + d) * 8));

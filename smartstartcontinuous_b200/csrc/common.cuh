@@ -117,6 +117,7 @@ struct ss_ctx {
     DevBuf kde_density, kde_ucb, kde_block_best, kde_result;
     bool kde_tc_attr_set = false;
     bool kde_result_clean = false;     // the counters in kde_result are zero (left so by the last completed call)
+    bool kde_fp64 = false;             // selections follow scipy's float64 evaluation (ss_kde_set_precision, kde_fp64.cu)
     // mapped pinned host memory the finish kernel writes the selection result to (+ completion flag)
     void* host_kde = nullptr;
     void* host_kde_dev = nullptr;

@@ -33,7 +33,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "common.cuh"
+#include "kde_shared.cuh"
 
 namespace {
 
@@ -500,21 +500,6 @@ kde_pairs_kernel(const float* __restrict__ pts, long long n_tiles, const float* 
 #include "kde_tc.cuh"
 
 // ---- 5. finish: slice reduction, fp64 rescue, density, UCB, arg-max --------------------
-struct KdeResult {
-    double best_ucb;
-    long long best_j;
-    unsigned int blocks_done;
-    int n_rescued;
-    unsigned int moments_ticket;      // last-block election of kde_moments_kernel
-    int pad;
-};
-
-// what a selection hands back to the host, written by the last block of kde_finish_kernel straight
-// into mapped pinned host memory (flag last, release at system scope): the call ends without a
-// device->host copy and without a stream synchronisation
-// the selection result in mapped pinned host memory: three tagged slots (common.cuh host_slot_put)
-constexpr int KDE_HOST_SLOTS = 3;     // best_ucb | best_j | (status, max_norm2_bits)
-
 __global__ void __launch_bounds__(256)
 kde_finish_kernel(const float* __restrict__ partial, int n_slices, long long m, long long m_pad,
                   const double* __restrict__ data, long long n, int d,
@@ -653,13 +638,6 @@ cudaError_t launch_pairs(ss_ctx* c, bool expanded, const float* pts, long long n
     return cudaGetLastError();
 }
 
-int pad_dim(int d) {
-    const int opts[] = {1, 2, 3, 4, 6, 8, 12, 16, 24, 32};
-    for (int o : opts)
-        if (d <= o) return o;
-    return -1;
-}
-
 }  // namespace
 
 // pair-stage variants, fastest first; a call starts optimistically with the fastest one its shape
@@ -691,10 +669,17 @@ int kde_exact_sums(ss_ctx* c, const double* data_dev, long long n, int d, double
     return SS_OK;
 }
 
+int kde_run_fp64(ss_ctx* c, const double* data_dev, long long n, int d, const double* queries_dev, long long m,
+                 const float* values_dev, long long n_transitions, double volume, double alpha, double beta,
+                 double* density_dev, double* ucb_dev, int64_t* out_best_j, double* out_best_ucb);
+
 int kde_run(ss_ctx* c, const double* data_dev, long long n, int d, const double* queries_dev,
             long long m, const float* values_dev, long long n_transitions, double volume,
             double alpha, double beta, double* density_dev, double* ucb_dev, int64_t* out_best_j,
             double* out_best_ucb, const double* running_sums) {
+    if (c->kde_fp64)     // SS_PRECISION_FP64 (kde_fp64.cu): fits from the data rows, never from running sums
+        return kde_run_fp64(c, data_dev, n, d, queries_dev, m, values_dev, n_transitions, volume, alpha, beta,
+                            density_dev, ucb_dev, out_best_j, out_best_ucb);
     const int D = pad_dim(d);
     if (D < 0) SS_FAIL(c, SS_EUNSUPPORTED, "kde: state dimension > 32 is not supported");
     const int mom_blocks = (int)std::min<long long>(c->sm_count * 2, (n + 255) / 256);

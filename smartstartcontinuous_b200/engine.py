@@ -162,6 +162,16 @@ class Engine:
             C.byref(best), C.byref(best_ucb)))
         return int(best.value), float(best_ucb.value), dens, ucb
 
+    def kde_set_precision(self, precision):
+        """Arithmetic of select_start / select_start_mirror / select_start_dev: "fp32" (default; densities to
+        ~1e-5) or "fp64" (scipy.stats.gaussian_kde's float64 evaluation operation for operation, alpha * values in
+        float32 like numpy: densities to ~1e-13, scipy's choice whenever the top-two UCB gap is larger).  Setting
+        the current value costs nothing."""
+        codes = {"fp32": PRECISION_FP32, "fp64": PRECISION_FP64}
+        if precision not in codes:
+            raise ValueError("selection precision must be 'fp32' or 'fp64', got %r" % (precision,))
+        self._check(self._lib.ss_kde_set_precision(self._h, codes[precision]))
+
     # NVLink peer-memory exchange for sharded batches (one process per GPU)
     def peer_setup(self, group=None):
         """Open the peer-memory exchange between the Engines of a torch.distributed group (one node,

@@ -70,10 +70,11 @@ class SmartStartContinuous(RLAgent):
                  nnd_mb_steps_per_rollout_train=333,
                  nnd_mb_steps_per_rollout_val=333,
 
-                 *, engine=None, device=0, nnd_mb_extra=None, device_mirror=True, value_net=None):
+                 *, engine=None, device=0, nnd_mb_extra=None, device_mirror=True, value_net=None,
+                 kde_precision="fp32"):
         self.param_dict = {k: v for k, v in locals().items()
                            if k not in ("self", "sess", "env", "agent", "engine", "nnd_mb_extra", "device_mirror", "value_net",
-                                        "__class__")}
+                                        "kde_precision", "__class__")}
         for name in ("self", "sess", "env", "__class__"):
             self.param_dict[name] = "Not serializable"
         self.param_dict["agent"] = agent.get_param_dict()
@@ -109,6 +110,11 @@ class SmartStartContinuous(RLAgent):
         # export the weights the agent has NOW), V = critic(q, actor(q)) is evaluated on the device in
         # front of the UCB and agent.get_state_value is not called for the candidates
         self.value_net = value_net
+        # arithmetic of the selection: "fp32" (default) or "fp64" (scipy's float64 evaluation, Engine.kde_set_precision);
+        # set on the engine before every selection, since the engine may be shared
+        if kde_precision not in ("fp32", "fp64"):
+            raise ValueError("kde_precision must be 'fp32' or 'fp64', got %r" % (kde_precision,))
+        self.kde_precision = kde_precision
 
         self.nnd_mb_agent = NND_MB_agent(
             env, sess, replay_buffer=self.replay_buffer,
@@ -173,6 +179,7 @@ class SmartStartContinuous(RLAgent):
             one_radii_volume = volume_of_n_dimensional_hyperellipsoid(self.nnd_mb_agent.radii)
         else:
             one_radii_volume = 1
+        self.engine.kde_set_precision(self.kde_precision)
         ring = self.replay_buffer.state_ring() if hasattr(self.replay_buffer, "state_ring") else None
         mirror = ring is not None and self.device_mirror
         values = None
