@@ -159,6 +159,9 @@ struct ss_ctx {
     DevBuf tc_w1, tc_w2, tc_w3, tc_misc, tc_b3;
     bool tc_ready = false;
     int tc_hp = 0;
+    // layer-1 layout the images were packed with (mpc_tc_prepare): state slots dz (action j -> input dz + j)
+    // and K slots k1.  The launchers and the device re-pack of ss_dyn_commit read it from here.
+    int tc_dz = 0, tc_k1 = 0;
     int tc_quad_clusters = -1;         // co-resident 4-CTA clusters of the small-batch kernel (-1: not probed)
     std::vector<std::vector<double>> hw, hb;   // host copies of the float64 parameters
     std::vector<DevBuf> w64, b64;      // padded float64 weights / biases (SS_PRECISION_FP64), same layout as w32 / b32

@@ -48,7 +48,7 @@ constexpr int NH = NC / 2;              // units of a chunk whose weights live i
 constexpr int KSLAB = 256;              // K elements per W2 stage (16 MMAs: amortises the issue loop)
 constexpr int STAGE_BYTES = NH * KSLAB * 2;   // 32 KB per CTA and stage
 constexpr int NSTAGE = 4;
-constexpr int K1_MAX = 32;              // K slots of the layer-1 MMA: 16 (d + da <= 4) or 32
+constexpr int K1_MAX = 32;              // K slots of the layer-1 MMA: 16 (3 (dz + da) + 2 <= 16) or 32
 constexpr int ACC_SLOTS = 2;
 constexpr int W1_CHUNK_BYTES_MAX = NH * K1_MAX * 2;   // 4 KB per CTA and chunk
 constexpr int A1_BYTES_MAX = TM * K1_MAX * 2;         // 8 KB
@@ -106,8 +106,12 @@ struct SmemT {
     static constexpr size_t END = TRACE;
 };
 
-// DT: register copies of the state (4 or 8); DZ: layer-3 outputs computed (>= d; 2, 3, 4 or 8);
-// K1T: K slots of the layer-1 MMA (16 when 3 (d + da) + 2 <= 16, else 32)
+// DT: register copies of the state (4 or 8); DZ: layer-3 outputs computed (>= d; 2, 3, 4 or 8), which is
+// also where the action inputs start (action j -> input DZ + j); K1T: K slots of the layer-1 MMA (16 when
+// 3 (DZ + da) + 2 <= 16, else 32).  DZ and K1T must be the dz_of / k1_slots the images were packed with
+// (ctx tc_dz / tc_k1): the launcher dispatches on exactly that pair, and every (d, da) that
+// mpc_tc_shape_supported accepts has an instantiation -- <4,2,16>, <4,2,32>, <4,3,16>, <4,3,32>,
+// <4,4,32>, <8,8,32> (tests/test_gpu_mpc_dims.py runs each against the float64 oracle).
 template <int DT, int DZ, int K1T>
 __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const RolloutArgs a, const Params p) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
@@ -600,11 +604,6 @@ static float bf16_val(uint16_t b) {
     return f;
 }
 
-static size_t smem_bytes(int d) {
-    const int dz = dz_of(d);
-    return (dz == 2 ? SmemT<2>::END : (dz <= 4 ? SmemT<4>::END : SmemT<8>::END)) + 128;
-}
-
 }  // namespace tc
 
 bool mpc_tc_shape_supported(const ss_ctx* c) {
@@ -678,6 +677,8 @@ int mpc_tc_prepare(ss_ctx* c) {
     SS_CUDA_CHECK(c, cudaMemcpyAsync(c->tc_w3.p, w3.data(), w3.size() * 4, cudaMemcpyHostToDevice, c->stream));
     SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
     c->tc_hp = hp;
+    c->tc_dz = dz;
+    c->tc_k1 = k1;
     c->tc_ready = true;
     return SS_OK;
 }
@@ -687,11 +688,11 @@ int mpc_tc_tile_rows() { return tc::TM; }
 // geometry of the operand images for ss_dyn_commit (dyn_train.cu), which re-packs them on the device
 void mpc_tc_geometry(const ss_ctx* c, int* k1, int* dz, int* hp, int* NC_, int* NH_, int* KSLAB_, int* CLUSTER_,
                      int* dzp) {
-    *k1 = tc::k1_slots(c->d, c->da);
-    *dz = tc::dz_of(c->d);
+    *k1 = c->tc_k1;
+    *dz = c->tc_dz;
     *hp = c->tc_hp;
     *NC_ = tc::NC; *NH_ = tc::NH; *KSLAB_ = tc::KSLAB; *CLUSTER_ = tc::CLUSTER;
-    *dzp = tc::w3_pair_floats(tc::dz_of(c->d)) / 2;
+    *dzp = tc::w3_pair_floats(c->tc_dz) / 2;
 }
 
 int mpc_tc_grid(const ss_ctx* c, long long tiles) {
@@ -727,12 +728,11 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
     const int grid = mpc_tc_grid(c, tile_count);
     if (grid_blocks_out) *grid_blocks_out = grid;
     p.iters = (int)((tile_count + grid - 1) / grid);
-    const size_t smem = smem_bytes(a.d) + (p.prof ? 3 * 256 * 8 : 0);
+    const size_t trace_bytes = p.prof ? 3 * 256 * 8 : 0;
     cudaLaunchConfig_t cfg;
     std::memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = smem;
     cfg.stream = c->stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -742,17 +742,22 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     cudaError_t e;
-    const int dz = dz_of(a.d), k1 = k1_slots(a.d, a.da);
+    // the instantiation whose input slots and W3 stride are the ones the images were packed with
+    const int dz = c->tc_dz, k1 = c->tc_k1;
 #define TC_LAUNCH(DT_, DZ_, K1_)                                                                              \
     do {                                                                                                      \
+        cfg.dynamicSmemBytes = SmemT<DZ_>::END + 128 + trace_bytes;                                          \
         e = cudaFuncSetAttribute(mpc_rollout_tc_kernel<DT_, DZ_, K1_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                 (int)smem);                                                                  \
+                                 (int)cfg.dynamicSmemBytes);                                                  \
         if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, mpc_rollout_tc_kernel<DT_, DZ_, K1_>, a, p);       \
     } while (0)
     if (dz == 2 && k1 == 16) TC_LAUNCH(4, 2, 16);          // e.g. MountainCar (d = 2, da = 1)
+    else if (dz == 2 && k1 == 32) TC_LAUNCH(4, 2, 32);     // d <= 2, da = 3 .. 8
     else if (dz == 3 && k1 == 16) TC_LAUNCH(4, 3, 16);     // e.g. Pendulum (d = 3, da = 1)
-    else if (dz <= 4) TC_LAUNCH(4, 4, 32);
-    else TC_LAUNCH(8, 8, 32);
+    else if (dz == 3 && k1 == 32) TC_LAUNCH(4, 3, 32);     // d = 3, da = 2 .. 7
+    else if (dz == 4 && k1 == 32) TC_LAUNCH(4, 4, 32);
+    else if (dz == 8 && k1 == 32) TC_LAUNCH(8, 8, 32);
+    else SS_FAIL(c, SS_EUNSUPPORTED, "mpc: no tcgen05 kernel for this layer-1 layout");
 #undef TC_LAUNCH
     if (e == cudaSuccess) e = cudaGetLastError();
     c->launches++;

@@ -45,8 +45,6 @@ constexpr uint32_t TMEM_COLS = 512, COL_H1 = 0, COL_ACC = 256;
 // D f32, A/B bf16, K-major, N = 128, M = 128 (cta_group::1)
 constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NC >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
 
-__host__ __device__ constexpr int dz_of(int d) { return d <= 2 ? 2 : (d <= 3 ? 3 : 4); }
-__host__ __device__ constexpr int k1_slots(int d, int da) { return 3 * (dz_of(d) + da) + 2 <= 16 ? 16 : 32; }
 __host__ __device__ constexpr int w3_pair_floats(int dz) { return dz <= 2 ? 4 : 8; }
 
 struct Params {
@@ -527,7 +525,8 @@ int mpc_tc_quad_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out) {
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     cudaError_t e;
-    const int dz = dz_of(a.d), k1 = k1_slots(a.d, a.da);
+    // the layout of the pair kernel's images (mpc_tc_prepare), instantiated for exactly that layout
+    const int dz = c->tc_dz, k1 = c->tc_k1;
 #define TCQ_LAUNCH(DT_, DZ_, K1_)                                                                                  \
     do {                                                                                                           \
         e = cudaFuncSetAttribute(mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
@@ -535,8 +534,11 @@ int mpc_tc_quad_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out) {
         if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_>, a, p);       \
     } while (0)
     if (dz == 2 && k1 == 16) TCQ_LAUNCH(4, 2, 16);
+    else if (dz == 2 && k1 == 32) TCQ_LAUNCH(4, 2, 32);
     else if (dz == 3 && k1 == 16) TCQ_LAUNCH(4, 3, 16);
-    else TCQ_LAUNCH(4, 4, 32);
+    else if (dz == 3 && k1 == 32) TCQ_LAUNCH(4, 3, 32);
+    else if (dz == 4 && k1 == 32) TCQ_LAUNCH(4, 4, 32);
+    else SS_FAIL(c, SS_EUNSUPPORTED, "mpc: no 4-CTA tcgen05 kernel for this layer-1 layout");
 #undef TCQ_LAUNCH
     if (e == cudaSuccess) e = cudaGetLastError();
     c->launches++;
