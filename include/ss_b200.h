@@ -217,6 +217,23 @@ int ss_mpc_replay(ss_ctx* ctx, int64_t k_global, double* out_sequence, double* o
  * for the winner's path): out_states [H+1, K_local, d], as do_forward_sim returns them
  * (dynamics_model.py:199-240). */
 int ss_mpc_get_states(ss_ctx* ctx, double* out_states);
+/* ss_mpc_forward_sim: Dyn_Model.do_forward_sim(many_in_parallel=True) (dynamics_model.py:204-240), no scoring.
+ * Needs ss_mpc_set_model only: no plan, and the caller's plan is left as it was.
+ *   start_states [n_starts, d] float64, host memory; n_starts = 1 (every sequence starts there: the reference's
+ *                [state, 0] form) or K (sequence k starts at row k).  A NaN or infinite start is SS_EINVAL (the
+ *                reference would carry it through every later state of that sequence).
+ *   actions      [K, H, da] float64, host or device memory (as ss_mpc_rollout)
+ *   precision    SS_PRECISION_AUTO / FP32 / BF16_TC / FP64, dispatched exactly as ss_mpc_rollout dispatches a
+ *                decision of the same K (pair vs quad kernel by the batch's tiles, thread vs CTA FP32 kernel)
+ *   out_states   [H+1, K, d] float64 (FP32 / BF16_TC: the FP32 rows widened, t = 0 is the start rounded to
+ *                float; FP64: the start rows exactly)
+ * Afterwards the context's last run is this simulation: ss_mpc_last_kernel reports its kernel and
+ * ss_mpc_get_states returns its states, while ss_mpc_finish, ss_mpc_finish_package, ss_mpc_replay and
+ * ss_mpc_projection_sums return SS_ESTATE until the next ss_mpc_rollout / ss_mpc_plan.  A decision after a
+ * forward simulation is bit-identical to the same decision without one.  SS_EINVAL: n_starts not 1 or K, K < 1,
+ * H < 1, a null pointer; SS_ESTATE: no model. */
+int ss_mpc_forward_sim(ss_ctx* ctx, const double* start_states, int64_t n_starts, int64_t K, int H,
+                       const double* actions, int precision, double* out_states);
 /* the device sampler alone: actions [K_local, H, da] for sequences k_offset.. (tests / oracle) */
 int ss_mpc_sample_actions(ss_ctx* ctx, int64_t K_local, int64_t k_offset, int H, int da,
                           uint64_t seed, const double* act_low, const double* act_high,

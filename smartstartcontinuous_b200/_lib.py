@@ -66,6 +66,8 @@ SIGNATURES = {
     "ss_mpc_finish_package": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), _c_int_p]),
     "ss_mpc_read_package": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "ss_mpc_get_states": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "ss_mpc_forward_sim": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                     C.c_void_p]),
     "ss_mpc_replay": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "ss_mpc_sample_actions": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_uint64,
                                         C.c_void_p, C.c_void_p, C.c_void_p]),

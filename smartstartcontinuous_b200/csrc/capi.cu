@@ -69,7 +69,8 @@ extern "C" int ss_destroy(ss_ctx* c) {
                       &c->mirror_stage, &c->value_net_params,
                       &c->tc_b3, &c->dyn_params, &c->dyn_m, &c->dyn_v, &c->dyn_x[0], &c->dyn_x[1], &c->dyn_z[0], &c->dyn_z[1],
                       &c->dyn_act, &c->dyn_scratch, &c->dyn_idx, &c->dyn_losses, &c->dyn_round,
-                      &c->plan_ds64, &c->plan_dl64, &c->mpc_states64, &c->mpc_scores64, &c->mpc_misc64};
+                      &c->plan_ds64, &c->plan_dl64, &c->mpc_states64, &c->mpc_scores64, &c->mpc_misc64,
+                      &c->fsim_plan, &c->fsim_plan64, &c->fsim_start};
     for (DevBuf* b : bufs) b->release();
     for (auto& b : c->w32) b.release();
     for (auto& b : c->b32) b.release();

@@ -193,8 +193,14 @@ struct ss_ctx {
     DevBuf mpc_states64, mpc_scores64, mpc_misc64;
     double gpow64_gamma = -1.0;
     int gpow64_T = 0;
+    // ss_mpc_forward_sim: the plan view its kernels score against (the caller's plan is neither needed nor
+    // touched), fp32 [ds 2 x SS_MAX_D | dl 2 | gamma^t fsim_plan_T] and the float64 twin, and the per-sequence
+    // start rows (fp32 [K][d] rounded from the caller's doubles, then float64 [K][d])
+    DevBuf fsim_plan, fsim_plan64, fsim_start;
+    int fsim_plan_T = 0;
     struct {
         bool valid = false;
+        bool forward_sim = false;      // the last run is a forward simulation: no decision to finish or replay
         int64_t K_local = 0, k_offset = 0, K_global = 0;
         int H = 0, wp_index = 0, penalty_mode = 0, precision = 0;
         double gamma = 0, hpf = 0;

@@ -147,7 +147,7 @@ __device__ void output_layer64(const double* __restrict__ in, int K_pad, const d
     }
 }
 
-template <int DT>
+template <int DT, bool ROWS>            // ROWS: per-sequence start rows (load_start)
 __global__ void __launch_bounds__(NT, 1) mpc_rollout_fp64_kernel(const Rollout64Args a) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
     extern __shared__ __align__(16) double sm64[];
@@ -169,9 +169,14 @@ __global__ void __launch_bounds__(NT, 1) mpc_rollout_fp64_kernel(const Rollout64
     ScoreAcc64 sc;
     if (owner) {
         double x[DT];
+        load_start<ROWS, DT>(a, live, k_local, x);
+        if constexpr (ROWS) {
 #pragma unroll
-        for (int j = 0; j < DT; ++j) x[j] = j < d ? a.state0[j] : 0.0;
-        for (int j = 0; j < d; ++j) st[j * SEQ + tid] = a.state0[j];
+            for (int j = 0; j < DT; ++j)
+                if (j < d) st[j * SEQ + tid] = x[j];
+        } else {
+            for (int j = 0; j < d; ++j) st[j * SEQ + tid] = a.state0[j];
+        }
         score_init64<DT>(a.plan, a.wp_index, x, sc);
     }
     for (int o = tid; o < a.din_pad * R; o += NT) actA[o] = 0.0;
@@ -256,8 +261,9 @@ __global__ void widen_kernel(const float* __restrict__ W, const float* __restric
 
 template <int DT>
 cudaError_t launch_fp64(ss_ctx* c, const Rollout64Args& a, int grid, size_t smem) {
-    cudaError_t e = cudaFuncSetAttribute(mpc_rollout_fp64_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) mpc_rollout_fp64_kernel<DT><<<grid, NT, smem, c->stream>>>(a);
+    auto kern = a.state0_rows ? mpc_rollout_fp64_kernel<DT, true> : mpc_rollout_fp64_kernel<DT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) kern<<<grid, NT, smem, c->stream>>>(a);
     return e;
 }
 

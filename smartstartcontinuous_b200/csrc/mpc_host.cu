@@ -90,6 +90,48 @@ Plan64 make_plan64(ss_ctx* c, double gamma, double hpf) {
     return p;
 }
 
+// Forward simulation: a two-waypoint plan of the context's own (waypoints 0 and 1, unit radii, gamma^t = 1, no
+// penalty) for the scoring code every rollout kernel runs.  Its scores are discarded; it only keeps the kernels
+// away from the caller's plan, which may not exist.
+constexpr int FSIM_GPOW = 2 * SS_MAX_D + 2;     // offset of gamma^t after [ds 2 x d | dl 2]
+
+template <typename T>
+int upload_fsim_plan(ss_ctx* c, DevBuf& buf, int T_steps) {
+    std::vector<T> v(FSIM_GPOW + T_steps, T(1));
+    for (int i = 0; i < 2 * SS_MAX_D; ++i) v[i] = i < c->d ? T(0) : T(1);     // ds rows 0 and 1 at stride d
+    v[2 * SS_MAX_D] = T(1);
+    v[2 * SS_MAX_D + 1] = T(0);
+    SS_CUDA_CHECK(c, buf.ensure(v.size() * sizeof(T)));
+    SS_CUDA_CHECK(c, cudaMemcpyAsync(buf.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+    SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+    return SS_OK;
+}
+
+PlanView fsim_plan_view(ss_ctx* c) {
+    PlanView p;
+    p.ds = c->fsim_plan.as<float>();
+    p.dl = p.ds + 2 * SS_MAX_D;
+    p.gpow = p.ds + FSIM_GPOW;
+    p.W = 2;
+    p.d = c->d;
+    for (int j = 0; j < SS_MAX_D; ++j) p.inv_r[j] = j < c->d ? 1.f : 0.f;
+    p.pen_scale = 0.f;
+    return p;
+}
+
+Plan64 fsim_plan64(ss_ctx* c) {
+    Plan64 p;
+    p.ds = c->fsim_plan64.as<double>();
+    p.dl = p.ds + 2 * SS_MAX_D;
+    p.gpow = p.ds + FSIM_GPOW;
+    p.W = 2;
+    p.d = c->d;
+    for (int j = 0; j < SS_MAX_D; ++j) p.r[j] = 1.0;
+    p.hpf = 0.0;
+    p.gamma = 0.0;
+    return p;
+}
+
 // float64 rows of the fp64 replay (after the gamma^t table)
 double* misc64_rows(ss_ctx* c) { return c->mpc_misc64.as<double>() + (c->run.H + 2) / 2 * 2; }
 
@@ -196,6 +238,7 @@ extern "C" int ss_mpc_set_model(ss_ctx* c, int d, int da, int num_fc_layers, int
     }
     c->model_set = true;
     c->run.valid = false;
+    c->fsim_plan_T = 0;                   // the forward-simulation plan's layout follows d
     c->tc_ready = false;
     if (mpc_tc_shape_supported(c)) {
         int rc = mpc_tc_prepare(c);
@@ -260,12 +303,25 @@ extern "C" int ss_mpc_sample_actions(ss_ctx* c, int64_t K_local, int64_t k_offse
 }
 
 static int reduce_projection_sums(ss_ctx* c, long long n_qcols);
+static int rollout_batch(ss_ctx* c, const double* actions, uint64_t seed, const double* act_low,
+                         const double* act_high, const float* start_rows, const double* start_rows64);
 
-// SS_PRECISION_FP64 rollout of the batch described by c->run (its actions already in place)
-static int rollout_fp64(ss_ctx* c, bool ref) {
+// SS_PRECISION_AUTO -> the kernel family the model shape allows; errors for an unknown or unavailable precision
+static int resolve_precision(ss_ctx* c, int& precision) {
+    if (precision == SS_PRECISION_AUTO) precision = c->tc_ready ? SS_PRECISION_BF16_TC : SS_PRECISION_FP32;
+    if (precision == SS_PRECISION_BF16_TC && !c->tc_ready)
+        SS_FAIL(c, SS_EUNSUPPORTED, "mpc: this model shape has no tcgen05 kernel (use precision FP32 or AUTO)");
+    if (precision != SS_PRECISION_FP32 && precision != SS_PRECISION_BF16_TC && precision != SS_PRECISION_FP64)
+        SS_FAIL(c, SS_EINVAL, "mpc: unknown precision");
+    return SS_OK;
+}
+
+// SS_PRECISION_FP64 rollout of the batch described by c->run (its actions already in place); start_rows:
+// per-sequence start states [K_local][d] on the device, or null
+static int rollout_fp64(ss_ctx* c, bool ref, const double* start_rows) {
     auto& r = c->run;
     const int T = r.H + 1, d = c->d;
-    if (c->gpow64_gamma != r.gamma || c->gpow64_T != T || !c->mpc_misc64.p) {
+    if (!r.forward_sim && (c->gpow64_gamma != r.gamma || c->gpow64_T != T || !c->mpc_misc64.p)) {
         std::vector<double> gp(T);
         for (int t = 0; t < T; ++t) gp[t] = std::pow(r.gamma, (double)t);     // gamma ** t (NND_MB_agent.py:611)
         // [gamma^t (T, padded to even) | replay rows T x (d + 1)]
@@ -279,8 +335,9 @@ static int rollout_fp64(ss_ctx* c, bool ref) {
     std::memset(&a, 0, sizeof(a));
     fill_model64_args(c, a);
     a.act = r.act;
-    a.plan = make_plan64(c, r.gamma, r.hpf);
+    a.plan = r.forward_sim ? fsim_plan64(c) : make_plan64(c, r.gamma, r.hpf);
     for (int j = 0; j < SS_MAX_D; ++j) a.state0[j] = r.state64[j];
+    a.state0_rows = start_rows;
     a.wp_index = r.wp_index; a.H = r.H; a.K_local = r.K_local; a.k_offset = r.k_offset;
     a.per_sample = !ref;
     SS_CUDA_CHECK(c, c->mpc_states64.ensure((size_t)T * r.K_local * (d + 1) * 8));
@@ -313,22 +370,33 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
         SS_FAIL(c, SS_EINVAL, "mpc: unknown penalty_mode");
     if (!actions && (!act_low || !act_high))
         SS_FAIL(c, SS_EINVAL, "mpc: device sampling needs act_low / act_high");
-    if (precision == SS_PRECISION_AUTO) precision = c->tc_ready ? SS_PRECISION_BF16_TC : SS_PRECISION_FP32;
-    if (precision == SS_PRECISION_BF16_TC && !c->tc_ready)
-        SS_FAIL(c, SS_EUNSUPPORTED, "mpc: this model shape has no tcgen05 kernel (use precision FP32 or AUTO)");
-    if (precision != SS_PRECISION_FP32 && precision != SS_PRECISION_BF16_TC && precision != SS_PRECISION_FP64)
-        SS_FAIL(c, SS_EINVAL, "mpc: unknown precision");
+    int rc = resolve_precision(c, precision);
+    if (rc) return rc;
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     timer_begin(c);
 
     auto& r = c->run;
     r.valid = false;
     r.finished = false;
+    r.forward_sim = false;
     r.K_local = K_local; r.k_offset = k_offset; r.K_global = K_global; r.H = H;
     r.wp_index = wp_index; r.penalty_mode = penalty_mode; r.precision = precision;
     r.gamma = gamma; r.hpf = hpf;
     for (int j = 0; j < SS_MAX_D; ++j) r.state[j] = j < c->d ? (float)state[j] : 0.f;
     for (int j = 0; j < SS_MAX_D; ++j) r.state64[j] = j < c->d ? state[j] : 0.0;
+    return rollout_batch(c, actions, seed, act_low, act_high, nullptr, nullptr);
+}
+
+// Sets up and launches the rollout of the batch c->run describes (ss_mpc_rollout and ss_mpc_forward_sim): action
+// upload, kernel dispatch, projection sums.  start_rows / start_rows64: per-sequence start states [K_local][d] on
+// the device for the precision's kernels, or null (every sequence starts at run.state).  A forward simulation
+// (run.forward_sim) scores against the context's own plan view and leaves the gamma^t tables of the decisions alone.
+static int rollout_batch(ss_ctx* c, const double* actions, uint64_t seed, const double* act_low,
+                         const double* act_high, const float* start_rows, const double* start_rows64) {
+    auto& r = c->run;
+    const int64_t K_local = r.K_local, k_offset = r.k_offset, K_global = r.K_global;
+    const int H = r.H, wp_index = r.wp_index, penalty_mode = r.penalty_mode, precision = r.precision;
+    const double gamma = r.gamma, hpf = r.hpf;
     int rc = fill_action_source(c, r.act, H, c->da, seed, act_low, act_high);
     if (rc) return rc;
     const int T = H + 1;
@@ -386,7 +454,7 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
         }
     }
     // gamma^t table (float64 pow, rounded once); re-uploaded only when gamma or the horizon change
-    if (c->gpow_gamma != gamma || c->gpow_T != T || !c->mpc_replay.p) {
+    if (!r.forward_sim && (c->gpow_gamma != gamma || c->gpow_T != T || !c->mpc_replay.p)) {
         std::vector<float> misc(T);
         for (int t = 0; t < T; ++t) misc[t] = (float)std::pow(gamma, (double)t);
         // [gamma^t (T) | pad | replay rows T x (d+1) | replay path T x d]
@@ -400,7 +468,7 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
     const bool ref = penalty_mode == SS_PENALTY_REFERENCE;
     r.states_stored = true;
     if (precision == SS_PRECISION_FP64) {
-        rc = rollout_fp64(c, ref);
+        rc = rollout_fp64(c, ref, start_rows64);
         if (rc) return rc;
         return reduce_projection_sums(c, mpc_fp64_grid(K_local));
     }
@@ -409,8 +477,9 @@ extern "C" int ss_mpc_rollout(ss_ctx* c, const double* state, int wp_index, int6
     std::memset(&a, 0, sizeof(a));
     fill_model_args(c, a);
     a.act = r.act;
-    a.plan = make_plan_view(c, gpow, gamma, hpf);
+    a.plan = r.forward_sim ? fsim_plan_view(c) : make_plan_view(c, gpow, gamma, hpf);
     for (int j = 0; j < SS_MAX_D; ++j) a.state0[j] = r.state[j];
+    a.state0_rows = start_rows;
     a.wp_index = wp_index; a.H = H; a.K_local = K_local; a.k_offset = k_offset;
     a.per_sample = penalty_mode == SS_PENALTY_PER_SAMPLE;
     SS_CUDA_CHECK(c, c->mpc_scores.ensure((size_t)K_local * 4));
@@ -502,7 +571,7 @@ static int reduce_projection_sums(ss_ctx* c, long long n_qcols) {
 
 extern "C" int ss_mpc_projection_sums(ss_ctx* c, double** sums_dev, int* count) {
     if (!c) return SS_EINVAL;
-    if (!c->run.valid) SS_FAIL(c, SS_ESTATE, "mpc: no rollout to take projection sums from");
+    if (!c->run.valid || c->run.forward_sim) SS_FAIL(c, SS_ESTATE, "mpc: no rollout to take projection sums from");
     if (c->run.penalty_mode != SS_PENALTY_REFERENCE) {
         if (sums_dev) *sums_dev = nullptr;
         if (count) *count = 0;
@@ -526,7 +595,7 @@ extern "C" int ss_mpc_projection_sums(ss_ctx* c, double** sums_dev, int* count) 
 // and the local winner's package at pkg_dst (and in mapped host memory when host_pkg is given)
 static int finish_device(ss_ctx* c, int want_path, double* pkg_dst, double* host_pkg, unsigned long long seq) {
     auto& r = c->run;
-    if (!r.valid) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish without ss_mpc_rollout");
+    if (!r.valid || r.forward_sim) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish without ss_mpc_rollout");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     const int T = r.H + 1;
     const float* gpow = c->mpc_replay.as<float>();
@@ -580,7 +649,7 @@ static void widen_scores(const std::vector<float>& sc, double* out_scores) {
 extern "C" int ss_mpc_finish(ss_ctx* c, int64_t* out_best_k, double* out_best_score, double* out_scores) {
     if (!c) return SS_EINVAL;
     auto& r = c->run;
-    if (!r.valid) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish without ss_mpc_rollout");
+    if (!r.valid || r.forward_sim) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish without ss_mpc_rollout");
     SS_CUDA_CHECK(c, c->mpc_package.ensure((size_t)package_count(c) * 8));
     int rc = finish_device(c, 0, c->mpc_package.as<double>(), nullptr, 0);
     if (rc) return rc;
@@ -604,7 +673,7 @@ static int reroll_winner(ss_ctx* c, int64_t k_global, float* rows_dev);
 extern "C" int ss_mpc_finish_package(ss_ctx* c, int want_path, double** package_dev, int* count) {
     if (!c) return SS_EINVAL;
     auto& r = c->run;
-    if (!r.valid) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish_package without ss_mpc_rollout");
+    if (!r.valid || r.forward_sim) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_finish_package without ss_mpc_rollout");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     const int n = package_count(c);
     SS_CUDA_CHECK(c, c->mpc_package.ensure((size_t)n * 8));
@@ -733,7 +802,7 @@ static int replay_path_fp64(ss_ctx* c, int64_t k_global, double* out_path) {
 extern "C" int ss_mpc_replay(ss_ctx* c, int64_t k_global, double* out_sequence, double* out_path) {
     if (!c) return SS_EINVAL;
     auto& r = c->run;
-    if (!r.valid) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_replay without ss_mpc_rollout");
+    if (!r.valid || r.forward_sim) SS_FAIL(c, SS_ESTATE, "mpc: ss_mpc_replay without ss_mpc_rollout");
     if (k_global < 0 || k_global >= r.K_global) SS_FAIL(c, SS_EINVAL, "mpc: replay index outside the batch");
     SS_CUDA_CHECK(c, cudaSetDevice(c->device));
     const int T = r.H + 1, d = c->d, da = c->da;
@@ -817,4 +886,59 @@ extern "C" int ss_mpc_plan(ss_ctx* c, const double* state, int wp_index, int64_t
     if (out_best_sequence) std::memcpy(out_best_sequence, pkg.data() + 2, (size_t)n_seq * 8);
     if (out_best_path) std::memcpy(out_best_path, pkg.data() + 2 + n_seq, (size_t)(H + 1) * c->d * 8);
     return SS_OK;
+}
+
+extern "C" int ss_mpc_forward_sim(ss_ctx* c, const double* start_states, int64_t n_starts, int64_t K, int H,
+                                  const double* actions, int precision, double* out_states) {
+    if (!c) return SS_EINVAL;
+    if (!c->model_set) SS_FAIL(c, SS_ESTATE, "mpc: set the model before a forward simulation");
+    if (!start_states || !actions || !out_states) SS_FAIL(c, SS_EINVAL, "mpc: null forward-simulation pointer");
+    if (K < 1 || H < 1) SS_FAIL(c, SS_EINVAL, "mpc: a forward simulation needs K >= 1 and H >= 1");
+    if (n_starts != 1 && n_starts != K) SS_FAIL(c, SS_EINVAL, "mpc: n_starts must be 1 or K");
+    const int d = c->d;
+    for (size_t i = 0; i < (size_t)n_starts * d; ++i)
+        if (!std::isfinite(start_states[i])) SS_FAIL(c, SS_EINVAL, "mpc: a start state is NaN or infinite");
+    int rc = resolve_precision(c, precision);
+    if (rc) return rc;
+    SS_CUDA_CHECK(c, cudaSetDevice(c->device));
+    timer_begin(c);
+
+    auto& r = c->run;
+    r.valid = false;
+    r.finished = false;
+    r.forward_sim = true;
+    r.K_local = K; r.k_offset = 0; r.K_global = K; r.H = H;
+    r.wp_index = 0; r.penalty_mode = SS_PENALTY_PER_SAMPLE; r.precision = precision;
+    r.gamma = 0.0; r.hpf = 0.0;
+    const bool per_row = n_starts > 1;
+    for (int j = 0; j < SS_MAX_D; ++j) r.state[j] = !per_row && j < d ? (float)start_states[j] : 0.f;
+    for (int j = 0; j < SS_MAX_D; ++j) r.state64[j] = !per_row && j < d ? start_states[j] : 0.0;
+    const bool f64 = precision == SS_PRECISION_FP64;
+    if (c->fsim_plan_T < H + 1) {
+        rc = f64 ? upload_fsim_plan<double>(c, c->fsim_plan64, H + 1) : upload_fsim_plan<float>(c, c->fsim_plan, H + 1);
+        if (rc) return rc;
+        rc = f64 ? upload_fsim_plan<float>(c, c->fsim_plan, H + 1) : upload_fsim_plan<double>(c, c->fsim_plan64, H + 1);
+        if (rc) return rc;
+        c->fsim_plan_T = H + 1;
+    }
+    // per-sequence starts: float64 rows as they are, or rounded to float as run.state is
+    std::vector<float> rows32;
+    const float* dev32 = nullptr;
+    const double* dev64 = nullptr;
+    if (per_row) {
+        const size_t n = (size_t)K * d;
+        SS_CUDA_CHECK(c, c->fsim_start.ensure(n * 8));
+        if (f64) {
+            SS_CUDA_CHECK(c, cudaMemcpyAsync(c->fsim_start.p, start_states, n * 8, cudaMemcpyHostToDevice, c->stream));
+            dev64 = c->fsim_start.as<double>();
+        } else {
+            rows32.resize(n);
+            for (size_t i = 0; i < n; ++i) rows32[i] = (float)start_states[i];
+            SS_CUDA_CHECK(c, cudaMemcpyAsync(c->fsim_start.p, rows32.data(), n * 4, cudaMemcpyHostToDevice, c->stream));
+            dev32 = c->fsim_start.as<float>();
+        }
+    }
+    rc = rollout_batch(c, actions, 0, nullptr, nullptr, dev32, dev64);
+    if (rc) return rc;
+    return ss_mpc_get_states(c, out_states);       // synchronises the stream (rows32 lives until then)
 }

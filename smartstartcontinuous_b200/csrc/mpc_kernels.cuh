@@ -25,6 +25,8 @@ struct RolloutArgs {
     float* scores_out;       // [K_local] (per-sample mode: final; reference mode: progress term)
     double* qsums;           // tcgen05 kernel, reference mode: [H+1][2][4 * tiles] a'.b' and b'.b' summed over the
                              // 32 rows of every (tile, row warp), or null (per-sample penalty)
+    const float* state0_rows;   // [K_local][d] per-sequence start states (forward simulation) or null: every
+                                // sequence starts at state0 (set: the launchers pick the kernels' ROWS = true)
 };
 
 // float64 rollout (mpc_fp64.cu): every operand and every operation in float64, the reference's element-wise
@@ -44,7 +46,26 @@ struct Rollout64Args {
     double* rows_out;        // [H+1][K_local][d + 1] (state, waypoint index after the move)
     double* scores_out;      // [K_local] (per-sample mode) or null
     double* qsums;           // reference mode: [H+1][2][ceil(K_local / 32)] a'.b' and b'.b' per 32 sequences, or null
+    const double* state0_rows;  // [K_local][d] per-sequence start states or null, as RolloutArgs::state0_rows
 };
+
+// Start state of sequence k_local, loaded once per sequence.  ROWS (a rollout kernel's template flag, set by the
+// launchers when state0_rows is given): a live sequence loads its own row, indexed by its batch-local k_local
+// (never a chunk-relative row), and a row that is not live (past K_local, a ragged last tile, a padding tile)
+// keeps zeros without reading the buffer, which has exactly K_local rows.  Otherwise every sequence starts at
+// state0.  Every thread that keeps a copy of a sequence's state calls this with the same (live, k_local).
+template <bool ROWS, int DT, typename T, typename A>
+__device__ __forceinline__ void load_start(const A& a, bool live, long long k_local, T (&x)[DT]) {
+    if constexpr (ROWS) {
+        const T* s = a.state0_rows + (size_t)k_local * a.d;
+#pragma unroll
+        for (int j = 0; j < DT; ++j) x[j] = live && j < a.d ? __ldg(s + j) : T(0);
+    } else {
+#pragma unroll
+        for (int j = 0; j < DT; ++j) x[j] = j < a.d ? a.state0[j] : T(0);
+    }
+}
+
 int mpc_fp64_launch(ss_ctx* c, const Rollout64Args& a);
 int mpc_fp64_grid(long long K_local);      // = projection-sum columns
 size_t mpc_fp64_smem_bytes(int din_pad, int h_pad);

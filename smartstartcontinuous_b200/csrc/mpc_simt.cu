@@ -136,8 +136,10 @@ __device__ void output_layer(const float* __restrict__ in, int K_pad, const floa
     __syncthreads();
 }
 
-template <int DT>
-__global__ void __launch_bounds__(ST) mpc_rollout_simt_kernel(const RolloutArgs a) {
+// ROWS: per-sequence start rows (load_start).  <4, ROWS> gets a minimum of one CTA per SM: left to its occupancy
+// heuristic, ptxas fits it into 80 registers and spills the scoring state inside the step loop.
+template <int DT, bool ROWS>
+__global__ void __launch_bounds__(ST, ROWS && DT == 4 ? 1 : 0) mpc_rollout_simt_kernel(const RolloutArgs a) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
     extern __shared__ __align__(16) float sm[];
     const int act_elems = (a.h_pad > a.din_pad ? a.h_pad : a.din_pad) * SR;
@@ -157,9 +159,14 @@ __global__ void __launch_bounds__(ST) mpc_rollout_simt_kernel(const RolloutArgs 
     ScoreAcc sc;
     float x[DT];
     if (owner) {
+        load_start<ROWS, DT>(a, live, k_local, x);
+        if constexpr (ROWS) {
 #pragma unroll
-        for (int j = 0; j < DT; ++j) x[j] = j < a.d ? a.state0[j] : 0.f;
-        for (int j = 0; j < a.d; ++j) st[j * SR + tid] = a.state0[j];
+            for (int j = 0; j < DT; ++j)
+                if (j < a.d) st[j * SR + tid] = x[j];
+        } else {
+            for (int j = 0; j < a.d; ++j) st[j * SR + tid] = a.state0[j];
+        }
         score_init<DT>(a.plan, a.wp_index, x, sc);
     }
     // zero the padded input rows once (rows d+da .. din_pad)
@@ -221,7 +228,7 @@ __global__ void __launch_bounds__(ST) mpc_rollout_simt_kernel(const RolloutArgs 
 // projection-sum table (32 consecutive sequences), so the tail and the multi-GPU exchange see the same layout.
 constexpr int TT = 128;                    // threads = sequences per CTA (4 warps = 4 table columns)
 
-template <int DT, int HP>                  // d <= DT, h_pad <= HP
+template <int DT, int HP, bool ROWS>       // d <= DT, h_pad <= HP; ROWS: per-sequence start rows (load_start)
 __global__ void __launch_bounds__(TT) mpc_rollout_thread_kernel(const RolloutArgs a) {
     pdl_trigger();
     extern __shared__ __align__(16) float sm[];
@@ -249,8 +256,7 @@ __global__ void __launch_bounds__(TT) mpc_rollout_thread_kernel(const RolloutArg
 
     ScoreAcc sc;
     float x[DT];
-#pragma unroll
-    for (int j = 0; j < DT; ++j) x[j] = j < a.d ? a.state0[j] : 0.f;
+    load_start<ROWS, DT>(a, live, k_local, x);
     score_init<DT>(a.plan, a.wp_index, x, sc);
 
     for (int t = 0; t < T; ++t) {
@@ -331,9 +337,18 @@ int mpc_simt_grid(const RolloutArgs& a) { return (int)((a.K_local + SR - 1) / SR
 
 bool mpc_simt_is_thread_kernel(const RolloutArgs& a) { return simt_thread_variant(a); }
 
+template <int DT>
+static cudaError_t launch_simt_kernel(ss_ctx* c, const RolloutArgs& a, int grid, size_t smem) {
+    auto kern = a.state0_rows ? mpc_rollout_simt_kernel<DT, true> : mpc_rollout_simt_kernel<DT, false>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) kern<<<grid, ST, smem, c->stream>>>(a);
+    return e;
+}
+
 template <int DT, int HP>
 static cudaError_t launch_thread_kernel(ss_ctx* c, const RolloutArgs& a, int grid, size_t smem) {
-    mpc_rollout_thread_kernel<DT, HP><<<grid, TT, smem, c->stream>>>(a);
+    if (a.state0_rows) mpc_rollout_thread_kernel<DT, HP, true><<<grid, TT, smem, c->stream>>>(a);
+    else mpc_rollout_thread_kernel<DT, HP, false><<<grid, TT, smem, c->stream>>>(a);
     return cudaGetLastError();
 }
 
@@ -354,20 +369,9 @@ int mpc_simt_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out) {
         SS_FAIL(c, SS_EUNSUPPORTED, "mpc: depth_fc_layers too large for the FP32 kernel's shared memory");
     const int grid = mpc_simt_grid(a);
     if (grid_blocks_out) *grid_blocks_out = grid;
-    cudaError_t e;
-    if (a.d <= 4) {
-        e = cudaFuncSetAttribute(mpc_rollout_simt_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)smem);
-        if (e == cudaSuccess) mpc_rollout_simt_kernel<4><<<grid, ST, smem, c->stream>>>(a);
-    } else if (a.d <= 8) {
-        e = cudaFuncSetAttribute(mpc_rollout_simt_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)smem);
-        if (e == cudaSuccess) mpc_rollout_simt_kernel<8><<<grid, ST, smem, c->stream>>>(a);
-    } else {
-        e = cudaFuncSetAttribute(mpc_rollout_simt_kernel<SS_MAX_D>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) mpc_rollout_simt_kernel<SS_MAX_D><<<grid, ST, smem, c->stream>>>(a);
-    }
+    cudaError_t e = a.d <= 4 ? launch_simt_kernel<4>(c, a, grid, smem)
+                  : a.d <= 8 ? launch_simt_kernel<8>(c, a, grid, smem)
+                             : launch_simt_kernel<SS_MAX_D>(c, a, grid, smem);
     if (e == cudaSuccess) e = cudaGetLastError();
     c->launches++;
     SS_CUDA_CHECK(c, e);

@@ -112,7 +112,8 @@ struct SmemT {
 // (ctx tc_dz / tc_k1): the launcher dispatches on exactly that pair, and every (d, da) that
 // mpc_tc_shape_supported accepts has an instantiation -- <4,2,16>, <4,2,32>, <4,3,16>, <4,3,32>,
 // <4,4,32>, <8,8,32> (tests/test_gpu_mpc_dims.py runs each against the float64 oracle).
-template <int DT, int DZ, int K1T>
+// ROWS: every sequence starts at its own row of a.state0_rows (load_start, forward simulation).
+template <int DT, int DZ, int K1T, bool ROWS = false>
 __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const RolloutArgs a, const Params p) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
     extern __shared__ __align__(128) unsigned char smem[];
@@ -214,8 +215,7 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
             // (critical path), ch 1 scores the trajectory in the shadow of the layer-2 MMAs
             float x[DT];
             ScoreAcc sc;
-#pragma unroll
-            for (int j = 0; j < DT; ++j) x[j] = j < a.d ? a.state0[j] : 0.f;
+            load_start<ROWS, DT>(a, live, k_local, x);
             if (ch == 1) score_init<DT>(a.plan, a.wp_index, x, sc);
             float act[SS_MAX_DA];
 #pragma unroll
@@ -747,9 +747,10 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
 #define TC_LAUNCH(DT_, DZ_, K1_)                                                                              \
     do {                                                                                                      \
         cfg.dynamicSmemBytes = SmemT<DZ_>::END + 128 + trace_bytes;                                          \
-        e = cudaFuncSetAttribute(mpc_rollout_tc_kernel<DT_, DZ_, K1_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                 (int)cfg.dynamicSmemBytes);                                                  \
-        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, mpc_rollout_tc_kernel<DT_, DZ_, K1_>, a, p);       \
+        auto kern = a.state0_rows ? mpc_rollout_tc_kernel<DT_, DZ_, K1_, true>                                \
+                                  : mpc_rollout_tc_kernel<DT_, DZ_, K1_, false>;                               \
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes); \
+        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, kern, a, p);                                       \
     } while (0)
     if (dz == 2 && k1 == 16) TC_LAUNCH(4, 2, 16);          // e.g. MountainCar (d = 2, da = 1)
     else if (dz == 2 && k1 == 32) TC_LAUNCH(4, 2, 32);     // d <= 2, da = 3 .. 8

@@ -76,7 +76,8 @@ struct Smem {
             p.prof[(trace_t - 10) * 64 + (ev)] = (unsigned long long)clock64();                   \
     } while (0)
 
-template <int DT, int DZ, int K1T>
+// ROWS: every sequence starts at its own row of a.state0_rows (load_start, forward simulation)
+template <int DT, int DZ, int K1T, bool ROWS = false>
 __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_quad_kernel(const RolloutArgs a, const Params p) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
     extern __shared__ __align__(128) unsigned char smem[];
@@ -188,8 +189,7 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_quad_kernel(const R
             const long long qcol = tile < p.tile_end ? tile * 4 + q : -1;
             float x[DT];
             ScoreAcc sc;
-#pragma unroll
-            for (int j = 0; j < DT; ++j) x[j] = j < a.d ? a.state0[j] : 0.f;
+            load_start<ROWS, DT>(a, live, k_local, x);     // every CTA of the cluster holds this tile's rows
             if (scorer) score_init<DT>(a.plan, a.wp_index, x, sc);
             float act[SS_MAX_DA];
 #pragma unroll
@@ -529,9 +529,10 @@ int mpc_tc_quad_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out) {
     const int dz = c->tc_dz, k1 = c->tc_k1;
 #define TCQ_LAUNCH(DT_, DZ_, K1_)                                                                                  \
     do {                                                                                                           \
-        e = cudaFuncSetAttribute(mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                 (int)smem);                                                                       \
-        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_>, a, p);       \
+        auto kern = a.state0_rows ? mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_, true>                                \
+                                  : mpc_rollout_tc_quad_kernel<DT_, DZ_, K1_, false>;                               \
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                     \
+        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, kern, a, p);                                            \
     } while (0)
     if (dz == 2 && k1 == 16) TCQ_LAUNCH(4, 2, 16);
     else if (dz == 2 && k1 == 32) TCQ_LAUNCH(4, 2, 32);

@@ -164,14 +164,28 @@ class Dyn_Model:
         return loss
 
     # ------------------------------------------------------------------ inference (engine)
-    def do_forward_sim(self, forwardsim_x_true, forwardsim_y, many_in_parallel):
+    def do_forward_sim(self, forwardsim_x_true, forwardsim_y, many_in_parallel, *, precision="fp32"):
         """Multi-step open-loop prediction (dynamics_model.py:199-270) on the GPU engine.
-        Returns a list of H+1 arrays [N, d] (parallel) or [d] (single sequence)."""
+        Returns a list of H+1 arrays [N, d] (parallel) or [d] (single sequence).
+
+        many_in_parallel, forwardsim_y = N action sequences [N, H, da]:
+          * len(forwardsim_x_true) == 2: the reference's [state, 0] form, forwardsim_x_true[0] starts every
+            sequence.  As in the reference, a [2, d] array of two start states takes this branch too: its first
+            row starts all N sequences.
+          * otherwise forwardsim_x_true holds the N start states ([N, d] array or a list of N arrays of length d),
+            sequence n starts at row n (multi-step prediction from many start states, e.g. k-step validation).
+            Any other shape raises ValueError.
+        precision: "fp32" (default), "bf16_tc", "auto" or "fp64" (the reference's float64 arithmetic)."""
         y = np.asarray(forwardsim_y, dtype=np.float64)
         if many_in_parallel:
-            if len(forwardsim_x_true) != 2:
-                raise ValueError("per-sequence start states are not supported by the engine rollout")
-            states = self.engine.forward_sim(forwardsim_x_true[0], y)
+            if len(forwardsim_x_true) == 2:
+                start = forwardsim_x_true[0]
+            else:
+                start = np.asarray(forwardsim_x_true, dtype=np.float64)
+                if start.ndim != 2 or y.ndim != 3 or start.shape != (y.shape[0], self.outputSize):
+                    raise ValueError("per-sequence start states must be [N, d] = [%s, %d], got shape %s"
+                                     % (y.shape[0] if y.ndim == 3 else "N", self.outputSize, start.shape))
+            states = self.engine.forward_sim(start, y, precision)
             return [states[t] for t in range(states.shape[0])]
-        states = self.engine.forward_sim(forwardsim_x_true[0], y[None, :, :])
+        states = self.engine.forward_sim(forwardsim_x_true[0], y[None, :, :], precision)
         return [states[t, 0] for t in range(states.shape[0])]

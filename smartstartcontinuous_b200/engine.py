@@ -385,8 +385,6 @@ class Engine:
         self._check(self._lib.ss_mpc_set_model(
             self._h, d, da, L, h, wp, bp, _ptr(n["mean_x"]), _ptr(n["std_x"]), _ptr(n["mean_y"]),
             _ptr(n["std_y"]), _ptr(n["mean_z"]), _ptr(n["std_z"])))
-        if self._model_shape is not None and self._model_shape[0] != d:
-            self._plan_set = False
         self._model_shape = (d, da, L, h)
 
     # ------------------------------------------------------------------ dynamics-model training (row f1)
@@ -464,7 +462,6 @@ class Engine:
             raise ValueError("desired_states [W, d], distances_left [W], radii [d] expected")
         self._check(self._lib.ss_mpc_set_plan(self._h, _ptr(ds), ds.shape[0], _ptr(dl), _ptr(r),
                                               ds.shape[1]))
-        self._plan_set = True
 
     def _plan_args(self, state, actions, K, H, act_low, act_high):
         d, da, _, _ = self._model_shape
@@ -598,14 +595,37 @@ class Engine:
         self._check(self._lib.ss_mpc_get_states(self._h, _ptr(out)))
         return out
 
-    def forward_sim(self, state, actions, precision="fp32"):
-        """Dyn_Model.do_forward_sim(many_in_parallel=True) on the GPU: [H+1, K, d] ("fp64": the reference's
-        float64 arithmetic)."""
-        if not getattr(self, "_plan_set", False):
-            d = self._model_shape[0]
-            self.set_plan(np.stack([np.zeros(d), np.ones(d)]), [1.0, 0.0], np.ones(d))
-        self.rollout(state, 0, actions=actions, penalty_mode="reference", precision=precision)
-        return self.get_states()
+    def forward_sim(self, state, actions=None, precision="fp32", *, actions_dev=None, K=None, H=None):
+        """Dyn_Model.do_forward_sim(many_in_parallel=True) on the GPU (ss_mpc_forward_sim): states [H+1, K, d].
+        state [d] starts every sequence there; [K, d] starts sequence k at row k.  actions [K, H, da], or
+        actions_dev = the device address of such samples (mt19937_uniform) with K and H given.  precision as in
+        plan ("fp64": the reference's float64 arithmetic).  Needs set_model only; the plan is neither needed nor
+        changed, and finish / replay / projection_sums_ptr refuse until the next rollout or plan."""
+        if self._model_shape is None:
+            raise RuntimeError("set_model() first")
+        d, da, _, _ = self._model_shape
+        st = _f64(state)
+        if st.ndim == 1 and st.shape[0] == d:
+            n_starts = 1
+        elif st.ndim == 2 and st.shape[1] == d:
+            n_starts = st.shape[0]
+        else:
+            raise ValueError("state must be [d] or [K, d] with d = %d, got shape %s" % (d, st.shape))
+        if actions_dev is not None:
+            actions = _DevicePointer(actions_dev)
+        elif actions is None:
+            raise ValueError("actions [K, H, da] or actions_dev are needed")
+        else:
+            actions = _f64(actions)
+            if actions.ndim != 3 or actions.shape[2] != da:
+                raise ValueError("actions must be [K, H, da]")
+            K, H = actions.shape[0], actions.shape[1]
+        K, H = int(K), int(H)
+        out = np.empty((H + 1, K, d))
+        self._check(self._lib.ss_mpc_forward_sim(self._h, _ptr(st), n_starts, K, H, _ptr(actions),
+                                                 _PRECISION[precision], _ptr(out)))
+        self._last = (K, H)
+        return out
 
     def replay(self, k_global):
         d, da, _, _ = self._model_shape
