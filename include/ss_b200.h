@@ -288,6 +288,10 @@ int ss_mpc_tc_supported(ss_ctx* ctx);
  * sequence (one hidden layer of <= 64 units, the reference's default 1 x 32 model), 4 = float64 (SS_PRECISION_FP64,
  * mpc_fp64.cu); -1 = none */
 int ss_mpc_last_kernel(ss_ctx* ctx);
+/* schedule of the last ss_mpc_rollout on the tcgen05 CTA-pair kernel: 0 = one tile per CTA at a time, 1 = two tiles
+ * per CTA offset by half a step (layouts with K1 = 16 and a padded hidden width of 512, at least two tiles per CTA;
+ * an odd last tile of a CTA still runs alone); -1 = the last rollout did not run that kernel */
+int ss_mpc_last_tc_schedule(ss_ctx* ctx);
 
 /* ---- dynamics-model training on the device (SURVEY 8f, row f1) ------------------------------
  * Replaces Dyn_Model.train (dynamics_model.py:52-171) as NND_MB_agent.train_dynamics_model calls it

@@ -73,6 +73,7 @@ SIGNATURES = {
                                         C.c_void_p, C.c_void_p, C.c_void_p]),
     "ss_mpc_tc_supported": (C.c_int, [C.c_void_p]),
     "ss_mpc_last_kernel": (C.c_int, [C.c_void_p]),
+    "ss_mpc_last_tc_schedule": (C.c_int, [C.c_void_p]),
     "ss_mt19937_uniform": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_int,
                                      C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "ss_mt19937_state": (C.c_int, [C.c_void_p, C.c_void_p, _c_int_p]),

@@ -209,6 +209,7 @@ struct ss_ctx {
         ActionSource act;
         bool states_stored = false;
         int kernel = 0;                // rollout kernel of this decision (ss_mpc_last_kernel)
+        int tc_schedule = -1;          // mpc_rollout_tc_kernel: 0 one tile per CTA, 1 two tiles (ss_mpc_last_tc_schedule)
         bool finished = false;         // the reference-mode penalty pass has rewritten the scores
         bool peer_sums = false;        // the projection sums were all-reduced over peer memory
         int sum_blocks = 0;

@@ -249,6 +249,9 @@ extern "C" int ss_mpc_set_model(ss_ctx* c, int d, int da, int num_fc_layers, int
 
 extern "C" int ss_mpc_tc_supported(ss_ctx* c) { return c && c->model_set && c->tc_ready ? 1 : 0; }
 extern "C" int ss_mpc_last_kernel(ss_ctx* c) { return c && c->run.valid ? c->run.kernel : -1; }
+extern "C" int ss_mpc_last_tc_schedule(ss_ctx* c) {
+    return c && c->run.valid && c->run.kernel == 1 ? c->run.tc_schedule : -1;
+}
 
 extern "C" int ss_mpc_set_plan(ss_ctx* c, const double* desired_states, int W,
                                const double* distances_left, const double* radii, int d) {

@@ -29,7 +29,9 @@
 // issues every MMA of the pair, warp-uniform loop, one elected lane; peer CTA: relays "my half of
 // the stage has landed" to the leader), warp 9 = TMA producer.
 // TMEM per CTA (512 columns): [0,256) H1 as bf16 A operand, [256,512) 2-deep ring of 128x128 FP32
-// accumulator chunks.  Cross-CTA signalling: mbarrier arrives on the leader's barriers
+// accumulator chunks.  Two-tile schedule (PAIR, hp = 512, K1 = 16): two tiles per CTA half a step apart, each with
+// H1 units 0-255 in TMEM and 256-511 in shared memory, so one tile's layer 2 covers the other's per-step chain.
+// Cross-CTA signalling: mbarrier arrives on the leader's barriers
 // (shared::cluster, release.cluster) and tcgen05.commit.cta_group::2 multicast to both CTAs.
 #include <cuda_bf16.h>
 
@@ -77,6 +79,7 @@ struct Params {
     int din;
     long long tile_begin, tile_end;     // this launch rolls the tiles [tile_begin, tile_end) of the batch
     int iters;                          // tile iterations per CTA (same for all: pair lock-step)
+    int pair_iters;                     // of these, iterations run two at a time (two-tile schedule)
     unsigned long long* prof;
 };
 
@@ -91,7 +94,29 @@ constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NC >
             trace_s[(trace_t - 10) * 256 + (ev)] = (unsigned long long)clock64();                  \
     } while (0)
 
-template <int DZ>
+// Two-tile schedule (PAIR): every CTA walks two tiles at once, offset by half a step.  TMEM holds K-slab 0
+// (units 0-255) of both tiles' H1 ([0,128) tile 0, [128,256) tile 1) and the two accumulator slots; K-slab 1
+// (units 256-511) of each tile's H1 is a K-major no-swizzle A image in shared memory.
+// W2 ring of the two-tile schedule: 4 x 16 KB (half a K-slab per stage).  Two 32 KB stages leave one stage of
+// lead, less than the latency of a 32 KB bulk copy from L2 at the 32 B/clk per SM that a busy tensor pipe consumes.
+constexpr int PAIR_STAGES = 4;
+constexpr int PSTAGE_BYTES = STAGE_BYTES / 2;
+constexpr int H1S_BYTES = TM * (HP_MAX - KSLAB) * 2;              // 64 KB: one tile's K-slab 1
+constexpr int PAIR_K1 = 16;                                       // layer-1 K slots the PAIR layout has room for
+constexpr int PAIR_BARS = 2 * PAIR_STAGES + 2 * ACC_SLOTS + 7;
+constexpr size_t SMEM_LIMIT = 232448;                             // 227 KiB of dynamic shared memory per CTA
+
+// two-tile schedule: stamps of half-steps 20-25 (steps 10-12 of both tiles of block 0's first tile pair), 64 per
+// half-step.  MMA warp: 2n+k before / 8+2n+k after the K-slab k of chunk n, 16 chunk-3 scratch free seen,
+// 17 chunk 2 issued, 18 / 19 before / after the waits for the other tile's layer 1.  Row warps (ch 0 at +20, ch 1 at +40): 0 start,
+// 1 other tile's step finished, 2 its x-split written, 3 scoring done, 4-6 epilogue n0-n2 done, 7 layer 1 converted.
+#define PAIR_TRACE(hs_, ev)                                                                               \
+    do {                                                                                                  \
+        if (p.prof && blockIdx.x == 0 && lane == 0 && (hs_) >= 20 && (hs_) < 26 && (ev) < 64)             \
+            trace_s[((hs_) - 20) * 64 + (ev)] = (unsigned long long)clock64();                            \
+    } while (0)
+
+template <int DZ, bool PAIR = false>
 struct SmemT {
     // dynamic shared memory carve-up (offsets in bytes from a 128-byte aligned base)
     static constexpr size_t W2_RING = 0;
@@ -105,6 +130,30 @@ struct SmemT {
     static constexpr size_t TRACE = TMEM_PTR + 16;     // SS_TC_TRACE stamps (only when tracing)
     static constexpr size_t END = TRACE;
 };
+// Layout of the kernels that run the two-tile schedule (K1 = 16 only).  The one-tile ring of a trailing
+// odd tile aliases the two H1 K-slab-1 images (the producer starts it only after the last two-tile MMA).
+template <int DZ>
+struct SmemT<DZ, true> {
+    static constexpr size_t H1S = 0;                                                  // 2 x 64 KB
+    static constexpr size_t W2_RING = 0;                                              // one-tile ring, 4 x 32 KB
+    static constexpr size_t PRING = H1S + 2 * (size_t)H1S_BYTES;                      // two-tile ring, 4 x 16 KB
+    static constexpr size_t W1 = PRING + (size_t)PAIR_STAGES * PSTAGE_BYTES;
+    static constexpr size_t A1 = W1 + (size_t)(HP_MAX / NC) * NH * PAIR_K1 * 2;       // 8 KB of W1
+    static constexpr size_t W3 = A1 + (size_t)TM * PAIR_K1 * 2;                       // one 4 KB A1 tile
+    static constexpr size_t ZX = W3 + (size_t)(HP_MAX / 2) * w3_pair_floats(DZ) * 4;
+    static constexpr size_t BARS = ZX + (size_t)TPR * TM * 8 * 4;
+    static constexpr int N_BARS = SmemT<DZ, false>::N_BARS + PAIR_BARS;
+    static constexpr size_t TMEM_PTR = BARS + (size_t)N_BARS * 8;
+    static constexpr size_t TRACE = TMEM_PTR + 16;
+    static constexpr size_t END = TRACE;
+    static_assert(NSTAGE * STAGE_BYTES <= 2 * H1S_BYTES, "the one-tile ring fits in the H1 images");
+    static_assert(END + 128 <= SMEM_LIMIT, "two-tile layout exceeds 227 KiB");
+};
+// (dz, K1) layouts whose two-tile layout fits: <4,2,16>, <4,3,16>.  <4,4,32> and <8,8,32> need 16 KB of W1 and
+// an 8 KB A1 tile (and <8,8,32> a 16 KB W3): they keep the one-tile schedule.
+__host__ __device__ constexpr bool pair_layout_fits(int dz, int k1) {
+    return k1 == PAIR_K1 && dz <= 3;
+}
 
 // DT: register copies of the state (4 or 8); DZ: layer-3 outputs computed (>= d; 2, 3, 4 or 8), which is
 // also where the action inputs start (action j -> input DZ + j); K1T: K slots of the layer-1 MMA (16 when
@@ -113,11 +162,14 @@ struct SmemT {
 // mpc_tc_shape_supported accepts has an instantiation -- <4,2,16>, <4,2,32>, <4,3,16>, <4,3,32>,
 // <4,4,32>, <8,8,32> (tests/test_gpu_mpc_dims.py runs each against the float64 oracle).
 // ROWS: every sequence starts at its own row of a.state0_rows (load_start, forward simulation).
-template <int DT, int DZ, int K1T, bool ROWS = false>
+// PAIR: the first 2 * p.pair_iters tile iterations run on the two-tile schedule (pair_layout_fits, hp = 512),
+// the rest on the one-tile schedule.
+template <int DT, int DZ, int K1T, bool ROWS = false, bool PAIR = false>
 __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const RolloutArgs a, const Params p) {
     pdl_trigger();      // the reduce / tail kernels behind this launch may be scheduled (they wait for its completion)
     extern __shared__ __align__(128) unsigned char smem[];
-    using Smem = SmemT<DZ>;
+    using Smem = SmemT<DZ, PAIR>;
+    static_assert(!PAIR || pair_layout_fits(DZ, K1T), "no two-tile layout for this instantiation");
     constexpr int MAXIN = (K1T - 2) / 3;            // network inputs the A tile has slots for
     constexpr int W1_CHUNK_BYTES = NH * K1T * 2;
     constexpr int DZP = w3_pair_floats(DZ) / 2;     // layer-3 outputs padded to 2 / 4 / 8
@@ -136,6 +188,18 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
     uint64_t* l1_full = h1_ready + HP_MAX / NC;         // local: layer-1 chunk complete (commit)
     uint64_t* x_ready = l1_full + HP_MAX / NC;          // leader's copy
     uint64_t* w1_full = x_ready + 1;                    // local
+    // two-tile schedule (PAIR): its own barriers, so the one-tile phases start fresh after it
+    uint64_t* p_w2_full = w1_full + 1;                  // [PAIR_STAGES] as w2_full
+    uint64_t* p_w2_empty = p_w2_full + PAIR_STAGES;     // [PAIR_STAGES] as w2_empty
+    uint64_t* p_acc_full = p_w2_empty + PAIR_STAGES;    // [ACC_SLOTS] layer-2 chunk complete
+    uint64_t* p_acc_free = p_acc_full + ACC_SLOTS;      // [ACC_SLOTS] leader's copy: slot drained (layer 2 or layer-1 chunk 1)
+    uint64_t* p_x_ready = p_acc_free + ACC_SLOTS;       // leader's copy: a tile's layer-1 A tile is in smem
+    uint64_t* p_l1a = p_x_ready + 1;                    // local: layer-1 chunks 0-2 of a tile complete
+    uint64_t* p_l1b = p_l1a + 1;                        // local: layer-1 chunk 3 complete
+    uint64_t* p_scr = p_l1b + 1;                        // leader's copy: chunk 2 loaded, its scratch columns are free
+    uint64_t* p_h1t = p_scr + 1;                        // leader's copy: H1 K-slab 0 (TMEM) converted
+    uint64_t* p_h1s = p_h1t + 1;                        // leader's copy: H1 K-slab 1 (smem) converted
+    uint64_t* p_n3a = p_h1s + 1;                        // local: K-slab 0 of a tile's last chunk complete
     uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem + Smem::TMEM_PTR);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -149,6 +213,11 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
     if (p.prof && blockIdx.x == 0 && tid == 0) {
         trace_clk0 = (unsigned long long)clock64();
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(trace_ns0));
+        if constexpr (PAIR) {
+            // kept in shared memory (2 stamps past the events) instead of 4 registers for the whole kernel
+            trace_s[3 * 256] = trace_clk0;
+            trace_s[3 * 256 + 1] = trace_ns0;
+        }
     }
     const int nch = p.hp / NC;          // accumulator chunks per layer
     const int nslab = p.hp / KSLAB;     // W2 K-slabs (stages) per chunk
@@ -156,6 +225,7 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
     constexpr int CPS = KSLAB / NC;     // layer-1 chunks per K-slab
     const uint32_t cta_rank = cluster_ctarank();
     const bool leader = cta_rank == 0;
+    const int it0 = PAIR ? 2 * p.pair_iters : 0;    // first tile iteration on the one-tile schedule
 
     // ---- one-time setup ----------------------------------------------------------------
     if (tid == 0) {
@@ -168,6 +238,17 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
         for (int c = 0; c < HP_MAX / NC; ++c) { mbar_init(&h1_ready[c], 2 * ROW_WARPS); mbar_init(&l1_full[c], 1); }
         mbar_init(x_ready, 2 * 4);       // the four ch-0 warps of each CTA
         mbar_init(w1_full, 1);
+        if constexpr (PAIR) {
+            for (int s = 0; s < PAIR_STAGES; ++s) { mbar_init(&p_w2_full[s], leader ? 2 : 1); mbar_init(&p_w2_empty[s], 1); }
+            for (int s = 0; s < ACC_SLOTS; ++s) { mbar_init(&p_acc_full[s], 1); mbar_init(&p_acc_free[s], 2 * ROW_WARPS); }
+            mbar_init(p_x_ready, 2 * 4);
+            mbar_init(p_l1a, 1);
+            mbar_init(p_l1b, 1);
+            mbar_init(p_scr, 2 * ROW_WARPS);
+            mbar_init(p_h1t, 2 * ROW_WARPS);
+            mbar_init(p_h1s, 2 * ROW_WARPS);
+            mbar_init(p_n3a, 1);
+        }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
@@ -205,7 +286,251 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
             upd_c[j] = j < a.d ? fmaf(__ldg(p.b3 + j), a.norm.std_z[j], a.norm.mean_z[j]) : 0.f;
             asm volatile("" : "+f"(upd_s[j]), "+f"(upd_c[j]));
         }
-        for (int it = 0; it < p.iters; ++it) {
+        if constexpr (PAIR) {
+            // ========================= ROW WARPS, two-tile schedule =========================
+            // Half-step h runs the layer 2 of tile x = h & 1 (step h >> 1); meanwhile these warps finish the
+            // other tile y's step (its last epilogue, exchange, update, scoring, x-split) and convert its next
+            // layer 1, which the MMA warp slots in between the two K-slabs of x's last chunk: chunk 0 in place
+            // in y's K-slab-0 columns, chunk 1 in accumulator slot 0, chunks 2 and 3 one after the other in x's
+            // K-slab-0 columns (dead once x's last chunk has read them) -> y's K-slab-1 image in smem.
+            // Per tile only what the step chain carries; the sequence index is recomputed from the tile pair
+            // and the Philox block of an action from its counter (no cached cursor): two tiles' state has to
+            // fit next to the conversion registers under the 168-register cap of 10 warps.
+            struct TileSt {
+                float x[DT];
+                ScoreAcc sc;
+                float act[MAXIN - DZ];          // K1T = 16: every action of the shape has an input slot
+            };
+            TileSt ts[2];
+            long long tile0 = 0;                // tile of ts[0]; ts[1] rolls tile0 + gridDim.x
+            auto k_of = [&](int i) { return (tile0 + (long long)i * gridDim.x) * TM + row; };
+            auto live_of = [&](int i) { return tile0 + (long long)i * gridDim.x < p.tile_end && k_of(i) < a.K_local; };
+            auto qcol_of = [&](int i) {
+                const long long tile = tile0 + (long long)i * gridDim.x;
+                return tile < p.tile_end ? tile * 4 + q : -1ll;
+            };
+            auto fetch_act = [&](int i, int t) {
+                ActionCursor cur;
+                action_cursor_init(cur);
+#pragma unroll
+                for (int j = 0; j < MAXIN - DZ; ++j)
+                    if (j < a.da) ts[i].act[j] = fetch_action_seq(a.act, cur, k_of(i), a.k_offset + k_of(i), t, j);
+            };
+            // layer-3 partial sums: only one tile has chunks in flight at a time (x's n0-n2, then its n3 first
+            // thing in the next half-step); zeroed right before n0, so they hold no register during scoring
+            float2 zacc[DZ];
+            const long long n_qcols = 4 * ((a.K_local + TM - 1) / TM);
+            unsigned char* h1s = smem + Smem::H1S;
+            auto xsplit = [&](TileSt& T) {
+                // as in the one-tile schedule: hi/lo split of the normalised (state, action) into A1
+                float xin[MAXIN];
+#pragma unroll
+                for (int j = 0; j < MAXIN; ++j) xin[j] = 0.f;
+#pragma unroll
+                for (int j = 0; j < DZ; ++j)
+                    if (j < MAXIN) xin[j] = (T.x[j] - a.norm.mean_x[j]) * a.norm.inv_std_x[j];
+#pragma unroll
+                for (int j = 0; j < MAXIN - DZ; ++j) xin[DZ + j] = (T.act[j] - a.norm.mean_y[j]) * a.norm.inv_std_y[j];
+                float slot[K1T];
+#pragma unroll
+                for (int s = 0; s < K1T; ++s) slot[s] = 0.f;
+#pragma unroll
+                for (int j = 0; j < MAXIN; ++j) {
+                    const float hi = bf16_hi(xin[j]);
+                    const float lo = xin[j] - hi;
+                    slot[3 * j] = hi;
+                    slot[3 * j + 1] = hi;
+                    slot[3 * j + 2] = lo;
+                }
+                slot[K1T - 2] = 1.f;
+                slot[K1T - 1] = 1.f;
+#pragma unroll
+                for (int kc = 0; kc < K1T / 8; ++kc) {
+                    uint4 v;
+                    v.x = pack_bf16(slot[8 * kc], slot[8 * kc + 1]);
+                    v.y = pack_bf16(slot[8 * kc + 2], slot[8 * kc + 3]);
+                    v.z = pack_bf16(slot[8 * kc + 4], slot[8 * kc + 5]);
+                    v.w = pack_bf16(slot[8 * kc + 6], slot[8 * kc + 7]);
+                    *reinterpret_cast<uint4*>(a1s + kc * (TM * 16) + row * 16) = v;
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                tc_fence_before();      // this warp's last tcgen05.ld of the scratch columns precedes layer 1
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(p_x_ready);
+            };
+            // layer-2 chunk n: relu + packed FFMA2 layer 3 into zacc
+            auto epilogue = [&](int n) {
+                const uint32_t slot_i = (uint32_t)(n & 1);
+                mbar_wait<false>(&p_acc_full[slot_i], (uint32_t)(n >> 1) & 1);
+                tc_fence_after();
+                uint32_t v0[32], v1[32];
+                tmem_ld32(lane_addr + COL_ACC + slot_i * NC + ch * CPT, v0);
+                tmem_ld32(lane_addr + COL_ACC + slot_i * NC + ch * CPT + 32, v1);
+                tmem_wait_ld();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(&p_acc_free[slot_i]);
+                const float* wrow = w3s + (size_t)((n * NC + ch * CPT) / 2) * (2 * DZP);
+#pragma unroll
+                for (int j2 = 0; j2 < CPT / 2; ++j2) {
+                    const uint32_t ua = j2 < 16 ? v0[(2 * j2) & 31] : v1[(2 * j2) & 31];
+                    const uint32_t ub = j2 < 16 ? v0[(2 * j2 + 1) & 31] : v1[(2 * j2 + 1) & 31];
+                    const float2 hh = make_float2(fmaxf(__uint_as_float(ua), 0.f), fmaxf(__uint_as_float(ub), 0.f));
+                    const float* wp = wrow + j2 * (2 * DZP);
+#pragma unroll
+                    for (int jq = 0; jq < DZP / 2; ++jq) {
+                        const float4 w = *reinterpret_cast<const float4*>(wp + 4 * jq);
+                        if (2 * jq < DZ) zacc[2 * jq] = __ffma2_rn(hh, make_float2(w.x, w.y), zacc[2 * jq]);
+                        if (2 * jq + 1 < DZ) zacc[2 * jq + 1] = __ffma2_rn(hh, make_float2(w.z, w.w), zacc[2 * jq + 1]);
+                    }
+                }
+            };
+            // last chunk, exchange of the two column halves, state update (same order as the one-tile schedule)
+            auto finish_step = [&](TileSt& T) {
+                epilogue(3);
+#pragma unroll
+                for (int j = 0; j < DZ; ++j) zx[(j * TPR + ch) * TM + row] = zacc[j].x + zacc[j].y;
+                asm volatile("bar.sync %0, 64;" ::"r"(2 + q) : "memory");
+#pragma unroll
+                for (int j = 0; j < DZ; ++j) {
+                    float zz = zx[(j * TPR) * TM + row];
+#pragma unroll
+                    for (int o = 1; o < TPR; ++o) zz += zx[(j * TPR + o) * TM + row];
+                    T.x[j] += fmaf(zz, upd_s[j], upd_c[j]);
+                }
+                asm volatile("bar.sync %0, 64;" ::"r"(2 + q) : "memory");   // zx is free for the other tile
+            };
+            // layer-1 chunk in TMEM -> relu, bf16 -> 8 K-groups of tile y's K-slab-1 image
+            auto to_smem = [&](const uint32_t (&v0)[32], const uint32_t (&v1)[32], int y, int c) {
+                unsigned char* img = h1s + (size_t)y * H1S_BYTES + row * 16;
+#pragma unroll
+                for (int g = 0; g < 8; ++g) {
+                    const uint32_t(&v)[32] = g < 4 ? v0 : v1;
+                    const int o = (g & 3) * 8;
+                    uint4 w;
+                    w.x = pack_bf16_relu(__uint_as_float(v[o + 0]), __uint_as_float(v[o + 1]));
+                    w.y = pack_bf16_relu(__uint_as_float(v[o + 2]), __uint_as_float(v[o + 3]));
+                    w.z = pack_bf16_relu(__uint_as_float(v[o + 4]), __uint_as_float(v[o + 5]));
+                    w.w = pack_bf16_relu(__uint_as_float(v[o + 6]), __uint_as_float(v[o + 7]));
+                    *reinterpret_cast<uint4*>(img + (size_t)((c - 2) * (NC / 8) + ch * (CPT / 8) + g) * (TM * 16)) = w;
+                }
+            };
+            auto convert_l1 = [&](int y, int scr, uint32_t ev) {
+                uint32_t v0[32], v1[32], pk0[16], pk1[16];
+                const uint32_t ycol = (uint32_t)y * (KSLAB / 2), scol = (uint32_t)scr * (KSLAB / 2);
+                mbar_wait<false>(p_l1a, ev & 1);
+                tc_fence_after();
+                // chunk 0: FP32 in y's K-slab-0 columns, converted in place (pair barrier: both threads loaded)
+                tmem_ld32(lane_addr + ycol + ch * CPT, v0);
+                tmem_ld32(lane_addr + ycol + ch * CPT + 32, v1);
+                tmem_wait_ld();
+                asm volatile("bar.sync %0, 64;" ::"r"(2 + q) : "memory");
+#pragma unroll
+                for (int c2 = 0; c2 < 16; ++c2) {
+                    pk0[c2] = pack_bf16_relu(__uint_as_float(v0[2 * c2]), __uint_as_float(v0[2 * c2 + 1]));
+                    pk1[c2] = pack_bf16_relu(__uint_as_float(v1[2 * c2]), __uint_as_float(v1[2 * c2 + 1]));
+                }
+                tmem_st16(lane_addr + ycol + ch * (CPT / 2), pk0);
+                tmem_st16(lane_addr + ycol + ch * (CPT / 2) + 16, pk1);
+                // chunk 1: FP32 in accumulator slot 0
+                tmem_ld32(lane_addr + COL_ACC + ch * CPT, v0);
+                tmem_ld32(lane_addr + COL_ACC + ch * CPT + 32, v1);
+                tmem_wait_ld();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(&p_acc_free[0]);
+#pragma unroll
+                for (int c2 = 0; c2 < 16; ++c2) {
+                    pk0[c2] = pack_bf16_relu(__uint_as_float(v0[2 * c2]), __uint_as_float(v0[2 * c2 + 1]));
+                    pk1[c2] = pack_bf16_relu(__uint_as_float(v1[2 * c2]), __uint_as_float(v1[2 * c2 + 1]));
+                }
+                tmem_st16(lane_addr + ycol + NC / 2 + ch * (CPT / 2), pk0);
+                tmem_st16(lane_addr + ycol + NC / 2 + ch * (CPT / 2) + 16, pk1);
+                tmem_wait_st();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(p_h1t);
+                // chunk 2: FP32 in x's K-slab-0 columns; once loaded they take chunk 3
+                tmem_ld32(lane_addr + scol + ch * CPT, v0);
+                tmem_ld32(lane_addr + scol + ch * CPT + 32, v1);
+                tmem_wait_ld();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(p_scr);
+                to_smem(v0, v1, y, 2);
+                mbar_wait<false>(p_l1b, ev & 1);
+                tc_fence_after();
+                tmem_ld32(lane_addr + scol + ch * CPT, v0);
+                tmem_ld32(lane_addr + scol + ch * CPT + 32, v1);
+                tmem_wait_ld();
+                to_smem(v0, v1, y, 3);
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic -> async proxy
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_leader(p_h1s);
+            };
+            uint32_t ev = 0;     // layer-1 events (one per tile and step, in the MMA warp's order)
+            int hs = 0;          // half-steps (SS_TC_TRACE)
+            const int tb = warp == 0 ? 20 : (warp == 4 ? 40 : 64);   // other warps are not stamped
+            for (int pit = 0; pit < p.pair_iters; ++pit) {
+#pragma unroll
+                tile0 = p.tile_begin + (long long)(2 * pit) * gridDim.x + blockIdx.x;
+#pragma unroll
+                for (int i = 0; i < 2; ++i) {
+                    TileSt& T = ts[i];
+                    load_start<ROWS, DT>(a, live_of(i), k_of(i), T.x);
+                    if (ch == 1) score_init<DT>(a.plan, a.wp_index, T.x, T.sc);
+#pragma unroll
+                    for (int j = 0; j < MAXIN - DZ; ++j) T.act[j] = 0.f;
+                    if (ch == 0 && live_of(i)) fetch_act(i, 0);
+                }
+                // tile 0's first layer 1 (scratch: tile 1's dead K-slab-0 columns)
+                if (ch == 0) xsplit(ts[0]);
+                convert_l1(0, 1, ev++);
+                for (int t = 0; t < a.H; ++t) {
+#pragma unroll
+                    for (int x = 0; x < 2; ++x) {
+                        const int y = 1 - x;
+                        TileSt& X = ts[x];
+                        TileSt& Y = ts[y];
+                        // tile y: the step whose layer 2 ran in the previous half-step
+                        PAIR_TRACE(hs, tb + 0);
+                        if (x == 1 || t > 0) {
+                            finish_step(Y);
+                            PAIR_TRACE(hs, tb + 1);
+                            if (x == 1 && t == a.H - 1 && ch == 1) {
+                                score_row<DT>(a, a.H, Y.x, Y.sc, live_of(y), k_of(y), qcol_of(y), n_qcols, lane);
+                                if (live_of(y) && a.scores_out) a.scores_out[k_of(y)] = Y.sc.score;
+                            }
+                        }
+                        const int tyn = x == 0 ? t : t + 1;     // tile y's next step
+                        if (tyn < a.H && ch == 0) {
+                            if (live_of(y) && tyn > 0) fetch_act(y, tyn);
+                            xsplit(Y);
+                        }
+                        PAIR_TRACE(hs, tb + 2);
+                        if (ch == 1) score_row<DT>(a, t, X.x, X.sc, live_of(x), k_of(x), qcol_of(x), n_qcols, lane);
+                        PAIR_TRACE(hs, tb + 3);
+#pragma unroll
+                        for (int j = 0; j < DZ; ++j) zacc[j] = make_float2(0.f, 0.f);
+#pragma unroll 1
+                        for (int n = 0; n < 3; ++n) {
+                            epilogue(n);
+                            PAIR_TRACE(hs, tb + 4 + n);
+                        }
+                        if (tyn < a.H) convert_l1(y, x, ev++);
+                        PAIR_TRACE(hs, tb + 7);
+                        ++hs;
+                    }
+                }
+                finish_step(ts[1]);
+                if (ch == 1) {
+                    score_row<DT>(a, a.H, ts[1].x, ts[1].sc, live_of(1), k_of(1), qcol_of(1), n_qcols, lane);
+                    if (live_of(1) && a.scores_out) a.scores_out[k_of(1)] = ts[1].sc.score;
+                }
+            }
+        }
+        for (int it = it0; it < p.iters; ++it) {
             const long long tile = p.tile_begin + (long long)it * gridDim.x + blockIdx.x;   // >= tile_end: padding
             const long long k_local = tile * TM + row;
             const bool live = tile < p.tile_end && k_local < a.K_local;
@@ -443,7 +768,127 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
                 l1_bar[c] = smem_u32(&l1_full[c]);
                 asm volatile("" : "+r"(l1_d[c]), "+r"(l1_bar[c]));
             }
-            for (int it = 0; it < p.iters; ++it) {
+            if constexpr (PAIR) {
+                // ====================== MMA ISSUER, two-tile schedule (hp = 512) ======================
+                // Static issue order of half-step h (tile x = h & 1 runs layer 2, tile y = 1 - x is one
+                // half-step behind):
+                //   x.n0 [slot 0] | x.n1 [slot 1] | x.n2 [slot 0] | x.n3 K-slab 0 [slot 1] |
+                //   y.L1 chunks 0, 1 [y slab 0, slot 0] | (x.n3 K-slab 0 complete) y.L1 chunk 2 [x slab 0] |
+                //   x.n3 K-slab 1 | (chunk 2 loaded) y.L1 chunk 3 [x slab 0]
+                // Layer 2: K-slab 0 of each chunk reads A from the tile's TMEM columns, K-slab 1 from its smem
+                // image (same K order as the one-tile schedule).  While x's chunks run, the row warps finish y's
+                // previous step and write y's layer-1 A tile; y's layer 1 then runs between the two K-slabs of
+                // x's last chunk, so its conversion hides under the 16 smem-A MMAs of that K-slab.
+                // Every write into TMEM columns that an earlier MMA reads or writes waits for that MMA's
+                // completion through an mbarrier: tcgen05.mma ops of one thread are ordered among themselves only
+                // when they share the accumulator, and chunk 2 overwrites x's K-slab 0 (A of x.n3 K-slab 0,
+                // accumulator slot 1) -- hence the commit on p_n3a.  y's slab 0 and slot 0 were last used by MMAs
+                // whose completion the row warps observed before they released x.n1's slot and x.n2's slot.
+                const uint32_t pring = smem_u32(smem + Smem::PRING), h1s_addr = smem_u32(smem + Smem::H1S);
+                uint32_t use0 = 0, use1 = 0;             // uses of accumulator slots 0 and 1 so far
+                uint32_t pw = 0, ev = 0, hs = 0;         // W2 blocks, layer-1 events, half-steps
+                auto take_slot = [&](int s) {
+                    uint32_t& u = s ? use1 : use0;      // s is a constant at every call: plain registers
+                    mbar_wait<true>(&p_acc_free[s], (u & 1) ^ 1);
+                    ++u;
+                };
+                auto l1_issue = [&](int c, uint32_t d) {
+#pragma unroll
+                    for (int ks = 0; ks < K1T / 16; ++ks) umma2_ss(d, l1_a[ks], l1_b[c][ks], IDESC, ks);
+                };
+                // chunks 0-2 of tile y's layer 1; scr: tile whose K-slab-0 columns take chunks 2 and 3 (after
+                // its last chunk's K-slab 0 has completed when wait_scr)
+                auto l1_first = [&](int y, int scr, bool wait_scr) {
+                    PAIR_TRACE(hs, 18);
+                    mbar_wait<true>(p_x_ready, ev & 1);
+                    take_slot(0);
+                    PAIR_TRACE(hs, 19);
+                    tc_fence_after();
+                    if (elect_one()) {
+                        l1_issue(0, tmem + (uint32_t)y * (KSLAB / 2));
+                        l1_issue(1, tmem + COL_ACC);
+                    }
+                    __syncwarp();
+                    if (wait_scr) {
+                        mbar_wait<true>(p_n3a, hs & 1);
+                        tc_fence_after();
+                    }
+                    PAIR_TRACE(hs, 17);
+                    if (elect_one()) {
+                        l1_issue(2, tmem + (uint32_t)scr * (KSLAB / 2));
+                        tc_commit_pair(p_l1a);
+                    }
+                    __syncwarp();
+                };
+                auto l1_last = [&](int scr) {
+                    mbar_wait<true>(p_scr, ev & 1);
+                    PAIR_TRACE(hs, 16);
+                    tc_fence_after();
+                    if (elect_one()) {
+                        l1_issue(3, tmem + (uint32_t)scr * (KSLAB / 2));
+                        tc_commit_pair(p_l1b);
+                    }
+                    __syncwarp();
+                    ++ev;
+                };
+                // K-slab ksl of chunk n: two 16 KB stages of 8 MMAs each
+                auto l2_slab = [&](int x, int n, int ksl) {
+                    PAIR_TRACE(hs, 2 * n + ksl);
+#pragma unroll
+                    for (int hf = 0; hf < 2; ++hf, ++pw) {
+                        const uint32_t st = pw % PAIR_STAGES;
+                        if (n == 0 && hf == 0)
+                            mbar_wait2(&p_w2_full[st], (pw / PAIR_STAGES) & 1, ksl ? p_h1s : p_h1t, hs & 1);
+                        else
+                            mbar_wait<true>(&p_w2_full[st], (pw / PAIR_STAGES) & 1);
+                        tc_fence_after();
+                        if (elect_one()) {
+                            const uint32_t d_tmem = tmem + COL_ACC + (uint32_t)(n & 1) * NC;
+                            const uint64_t b0 = make_desc(pring + st * PSTAGE_BYTES, NH);
+                            if (ksl == 0) {
+#pragma unroll
+                                for (int ks = 0; ks < KSLAB / 32; ++ks)
+                                    umma2_ts(d_tmem, tmem + (uint32_t)x * (KSLAB / 2) + (hf * KSLAB / 32 + ks) * 8,
+                                             b0 + (uint64_t)((ks * 2 * (NH * 16)) >> 4), IDESC, (hf | ks) != 0);
+                            } else {
+                                const uint64_t a0 = make_desc(h1s_addr + (uint32_t)x * H1S_BYTES, TM);
+#pragma unroll
+                                for (int ks = 0; ks < KSLAB / 32; ++ks)
+                                    umma2_ss(d_tmem, a0 + (uint64_t)(((hf * KSLAB / 32 + ks) * 2 * (TM * 16)) >> 4),
+                                             b0 + (uint64_t)((ks * 2 * (NH * 16)) >> 4), IDESC, 1u);
+                            }
+                            tc_commit_pair(&p_w2_empty[st]);
+                            if (ksl == 1 && hf == 1) tc_commit_pair(&p_acc_full[n & 1]);
+                            if (n == 3 && ksl == 0 && hf == 1) tc_commit_pair(p_n3a);
+                        }
+                        __syncwarp();
+                    }
+                    PAIR_TRACE(hs, 8 + 2 * n + ksl);
+                };
+                for (int pit = 0; pit < p.pair_iters; ++pit) {
+                    l1_first(0, 1, false);      // tile 1's columns: last read by MMAs the rows saw complete
+                    l1_last(1);
+                    for (int t = 0; t < a.H; ++t) {
+#pragma unroll
+                        for (int x = 0; x < 2; ++x) {
+                            const bool y_next = x == 0 || t + 1 < a.H;
+#pragma unroll
+                            for (int n = 0; n < 3; ++n) {
+                                take_slot(n & 1);
+                                l2_slab(x, n, 0);
+                                l2_slab(x, n, 1);
+                            }
+                            take_slot(1);
+                            l2_slab(x, 3, 0);
+                            if (y_next) l1_first(1 - x, x, true);
+                            l2_slab(x, 3, 1);
+                            if (y_next) l1_last(x);
+                            ++hs;
+                        }
+                    }
+                }
+            }
+            for (int it = it0; it < p.iters; ++it) {
                 for (int t = 0; t < a.H; ++t, ++step_it) {
                     const int trace_it = it, trace_t = t;
                     // layer 1: chunk c = A1 [256 x K1T] * W1img[c] [128 x K1T]^T; odd chunks go to the
@@ -542,8 +987,16 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
             // ============================ STAGE RELAY (peer CTA) ===============================
             // tell the leader's MMA warp when this CTA's half of a W2 stage has landed
             if (lane == 0) {
+                if constexpr (PAIR) {
+                    const long long ptotal = (long long)p.pair_iters * 2 * a.H * nch * nslab * 2;
+                    for (long long i = 0; i < ptotal; ++i) {
+                        const uint32_t st = (uint32_t)(i % PAIR_STAGES);
+                        mbar_wait<false>(&p_w2_full[st], (uint32_t)(i / PAIR_STAGES) & 1);
+                        mbar_arrive_leader(&p_w2_full[st]);
+                    }
+                }
                 uint32_t w2_it = 0;
-                const long long total = (long long)p.iters * a.H * nch * nslab;
+                const long long total = (long long)(p.iters - it0) * a.H * nch * nslab;
                 for (long long i = 0; i < total; ++i, ++w2_it) {
                     const uint32_t st = w2_it % NSTAGE;
                     mbar_wait<false>(&w2_full[st], (w2_it / NSTAGE) & 1);
@@ -554,9 +1007,27 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
     } else {
         // =============================== TMA PRODUCER =====================================
         if (lane == 0) {
-            uint32_t w2_it = 0;
             const int blocks = nch * nslab;
-            for (int it = 0; it < p.iters; ++it)
+            if constexpr (PAIR) {
+                // the two-tile stream: one W2 pass per half-step in the MMA warp's issue order, each 32 KB block
+                // as two 16 KB stages (K 0-127, K 128-255 of the slab: contiguous in the K-major image)
+                const long long ptotal = (long long)p.pair_iters * 2 * a.H * blocks * 2;
+                for (long long i = 0; i < ptotal; ++i) {
+                    const uint32_t st = (uint32_t)(i % PAIR_STAGES);
+                    const long long blk = (i >> 1) % blocks;
+                    mbar_wait<false>(&p_w2_empty[st], ((uint32_t)(i / PAIR_STAGES) & 1) ^ 1);
+                    mbar_expect_tx(&p_w2_full[st], PSTAGE_BYTES);
+                    bulk_g2s(smem + Smem::PRING + (size_t)st * PSTAGE_BYTES,
+                             reinterpret_cast<const unsigned char*>(p.w2_img) +
+                                 ((size_t)blk * CLUSTER + cta_rank) * STAGE_BYTES + (size_t)(i & 1) * PSTAGE_BYTES,
+                             PSTAGE_BYTES, &p_w2_full[st]);
+                }
+                // the one-tile ring overwrites the H1 images: wait for the last two-tile MMA (in-order completion)
+                for (long long i = ptotal - PAIR_STAGES; i < ptotal; ++i)
+                    if (i >= 0) mbar_wait<false>(&p_w2_empty[i % PAIR_STAGES], (uint32_t)(i / PAIR_STAGES) & 1);
+            }
+            uint32_t w2_it = 0;
+            for (int it = it0; it < p.iters; ++it)
                 for (int t = 0; t < a.H; ++t)
                     for (int blk = 0; blk < blocks; ++blk, ++w2_it) {
                         const uint32_t st = w2_it % NSTAGE;
@@ -581,6 +1052,10 @@ __global__ void __launch_bounds__(THREADS, 1) mpc_rollout_tc_kernel(const Rollou
             // SM clock actually delivered over the kernel: cycles / globaltimer nanoseconds
             unsigned long long ns1;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
+            if constexpr (PAIR) {
+                trace_clk0 = trace_s[3 * 256];
+                trace_ns0 = trace_s[3 * 256 + 1];
+            }
             p.prof[3 * 256] = (unsigned long long)clock64() - trace_clk0;
             p.prof[3 * 256 + 1] = ns1 - trace_ns0;
         }
@@ -728,6 +1203,13 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
     const int grid = mpc_tc_grid(c, tile_count);
     if (grid_blocks_out) *grid_blocks_out = grid;
     p.iters = (int)((tile_count + grid - 1) / grid);
+    // two-tile schedule: tiles go to a CTA two at a time, an odd last one runs on the one-tile schedule.
+    // SS_TC_PAIR=0 forces the one-tile schedule (tests compare the two).
+    const char* pair_env = getenv("SS_TC_PAIR");
+    const bool pair = pair_layout_fits(c->tc_dz, c->tc_k1) && c->tc_hp == HP_MAX && p.iters >= 2 &&
+                      !(pair_env && std::atoi(pair_env) == 0);
+    p.pair_iters = pair ? p.iters / 2 : 0;
+    c->run.tc_schedule = pair ? 1 : 0;
     const size_t trace_bytes = p.prof ? 3 * 256 * 8 : 0;
     cudaLaunchConfig_t cfg;
     std::memset(&cfg, 0, sizeof(cfg));
@@ -752,7 +1234,17 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
         e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes); \
         if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, kern, a, p);                                       \
     } while (0)
-    if (dz == 2 && k1 == 16) TC_LAUNCH(4, 2, 16);          // e.g. MountainCar (d = 2, da = 1)
+#define TC_LAUNCH_PAIR(DT_, DZ_, K1_)                                                                         \
+    do {                                                                                                      \
+        cfg.dynamicSmemBytes = SmemT<DZ_, true>::END + 128 + (trace_bytes ? trace_bytes + 16 : 0);            \
+        auto kern = a.state0_rows ? mpc_rollout_tc_kernel<DT_, DZ_, K1_, true, true>                          \
+                                  : mpc_rollout_tc_kernel<DT_, DZ_, K1_, false, true>;                         \
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes); \
+        if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, kern, a, p);                                       \
+    } while (0)
+    if (pair && dz == 2) TC_LAUNCH_PAIR(4, 2, 16);
+    else if (pair && dz == 3) TC_LAUNCH_PAIR(4, 3, 16);
+    else if (dz == 2 && k1 == 16) TC_LAUNCH(4, 2, 16);     // e.g. MountainCar (d = 2, da = 1)
     else if (dz == 2 && k1 == 32) TC_LAUNCH(4, 2, 32);     // d <= 2, da = 3 .. 8
     else if (dz == 3 && k1 == 16) TC_LAUNCH(4, 3, 16);     // e.g. Pendulum (d = 3, da = 1)
     else if (dz == 3 && k1 == 32) TC_LAUNCH(4, 3, 32);     // d = 3, da = 2 .. 7
@@ -760,10 +1252,28 @@ int mpc_tc_launch(ss_ctx* c, const RolloutArgs& a, int* grid_blocks_out, long lo
     else if (dz == 8 && k1 == 32) TC_LAUNCH(8, 8, 32);
     else SS_FAIL(c, SS_EUNSUPPORTED, "mpc: no tcgen05 kernel for this layer-1 layout");
 #undef TC_LAUNCH
+#undef TC_LAUNCH_PAIR
     if (e == cudaSuccess) e = cudaGetLastError();
     c->launches++;
     SS_CUDA_CHECK(c, e);
-    if (p.prof) {
+    if (p.prof && pair) {
+        std::vector<unsigned long long> h(3 * 256 + 2);
+        SS_CUDA_CHECK(c, cudaMemcpyAsync(h.data(), p.prof, h.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+        SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));
+        fprintf(stderr, "[trace] block 0: %llu clk in %llu ns = %.0f MHz delivered SM clock (two-tile schedule)\n",
+                h[3 * 256], h[3 * 256 + 1], h[3 * 256 + 1] ? 1e3 * (double)h[3 * 256] / (double)h[3 * 256 + 1] : 0.0);
+        const unsigned long long t0 = h[0];
+        for (int hs = 0; hs < 6; ++hs) {
+            fprintf(stderr, "[trace half-step %d: tile %d layer 2, tile %d finishing] mma", 20 + hs, hs & 1, 1 - (hs & 1));
+            for (int e = 0; e < 20; ++e) fprintf(stderr, " %d:%lld", e, h[hs * 64 + e] ? (long long)(h[hs * 64 + e] - t0) : -1);
+            for (int w = 20; w <= 40; w += 20) {
+                fprintf(stderr, " | ch%d", w / 20 - 1);
+                for (int e = 0; e < 8; ++e)
+                    fprintf(stderr, " %d:%lld", e, h[hs * 64 + w + e] ? (long long)(h[hs * 64 + w + e] - t0) : -1);
+            }
+            fprintf(stderr, "\n");
+        }
+    } else if (p.prof) {
         std::vector<unsigned long long> h(3 * 256 + 2);
         SS_CUDA_CHECK(c, cudaMemcpyAsync(h.data(), p.prof, h.size() * 8, cudaMemcpyDeviceToHost, c->stream));
         SS_CUDA_CHECK(c, cudaStreamSynchronize(c->stream));

@@ -454,6 +454,10 @@ class Engine:
                 3: "mpc_rollout_thread_kernel", 4: "mpc_rollout_fp64_kernel"}.get(
             int(self._lib.ss_mpc_last_kernel(self._h)))
 
+    def last_tc_schedule(self):
+        """Schedule of the last rollout on mpc_rollout_tc_kernel: "one_tile", "two_tile", or None."""
+        return {0: "one_tile", 1: "two_tile"}.get(int(self._lib.ss_mpc_last_tc_schedule(self._h)))
+
     def set_plan(self, desired_states, distances_left, radii):
         ds = _f64(desired_states)
         dl = _f64(distances_left).reshape(-1)
